@@ -42,17 +42,30 @@ N > 1 (torchrun, one rank per GPU; ``scaling: strong``)
 ``kernels_numba.update_coefficients`` + ``ExpectationMaximization`` normalisations, numpy when
 numba is missing), one process per run like its spawn pool (src/mmsbm.py:182-185), on a bounded
 row sample; rank 0 only.
+
+``--dump-outputs DIR`` (N = 1) writes what the timed ``Engine.run`` loop left after its last step,
+as a caller reads it back with ``Engine.get_params``: DIR/theta.npy [S,U,K], DIR/eta.npy [S,I,L]
+and DIR/pr.npy [S,K,L,R], float64.  An array above a third of 64 MB keeps a fixed sample of its
+id axis (rows drawn with seed 0, sorted; the same rows for the same shape), so that the outputs of
+two builds on the same arguments can be compared element for element.  The ml1m_cv workload
+writes DIR/cv_accuracies.npy.
+
+The benchmark writes nothing into the source tree: it runs in a temporary working directory (the
+MMSBM logger writes mmsbm.log into the working directory) and writes no bytecode.
 """
 import argparse
+import contextlib
 import ctypes
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -116,6 +129,24 @@ def child_seeds(n):
 def b_alg(U, I, N, K, L, S):
     """Algorithmic bytes per rating-update, SURVEY.md section 8(d)."""
     return 8.0 * (K + L) + 16.0 / S + 16.0 * (K * U + L * I) / N
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, arrays, id_axis=1):
+    """Write each array as out_dir/<name>.npy (float64).  One larger than DUMP_BYTES / len(arrays)
+    keeps a fixed, seeded sample of its ``id_axis`` so that all files together stay within
+    DUMP_BYTES."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 4096                  # room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64)
+        if a.nbytes > share:
+            per_row = a.nbytes // a.shape[id_axis]
+            rows = np.sort(np.random.default_rng(0).choice(a.shape[id_axis], share // per_row, replace=False))
+            a = np.take(a, rows, axis=id_axis)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
 
 
 def _json(path):
@@ -492,15 +523,19 @@ def run_single(args, shape, cx):
     eng.set_params(th0, et0, pr0)
 
     clocks = ClockSampler(cx.local_rank)
-    launches0 = _lib.launch_count()
-    for _ in range(args.warmup):
-        eng.run(T)
-    cx.barrier()
-    launches1 = _lib.launch_count()
-    ms = cx.timed(lambda: eng.run(T), args.steps, 0)
-    launches = _lib.launch_count() - launches1
-    clk = clocks.stop()
-    del launches0
+    try:
+        for _ in range(args.warmup):
+            eng.run(T)
+        cx.barrier()
+        launches1 = _lib.launch_count()
+        ms = cx.timed(lambda: eng.run(T), args.steps, 0)
+        launches = _lib.launch_count() - launches1
+    finally:
+        clk = clocks.stop()
+    if args.dump_outputs:                       # before kernel_times, which steps the engine further
+        th, et, pr = eng.get_params()
+        dump_outputs(args.dump_outputs, {"theta": th, "eta": et, "pr": pr})
+        del th, et, pr
     value = float(N) * T * S * args.steps / (ms * 1e-3)
     ms_it = ms / args.steps / T
 
@@ -723,12 +758,14 @@ def run_multi(args, shape, cx):
     clocks = ClockSampler(cx.local_rank)
     modes = {}
     want = [m for m in ("runs", "sharded") if args.mode in ("best", m)]
-    for mode in want:
-        if mode == "runs":
-            modes[mode] = runs_record(cx, data, shape, T, args.steps, args.warmup)
-        else:
-            modes[mode] = sharded_record(cx, data, shape, T, args.steps, args.warmup, check_single_gpu=False)
-    clk = clocks.stop()
+    try:
+        for mode in want:
+            if mode == "runs":
+                modes[mode] = runs_record(cx, data, shape, T, args.steps, args.warmup)
+            else:
+                modes[mode] = sharded_record(cx, data, shape, T, args.steps, args.warmup, check_single_gpu=False)
+    finally:
+        clk = clocks.stop()
     best = max(modes, key=lambda m: modes[m]["value"])
     b = modes[best]
     e2e = None if args.no_e2e else e2e_multi(cx, data, shape, T, best, min(args.steps, 3))
@@ -802,6 +839,8 @@ def run_cv(args, shape, cx):
         dt = cx.max_over_ranks(time.perf_counter() - t0)
         if k >= args.warmup:
             times.append(dt)
+    if cx.rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"cv_accuracies": np.asarray(acc, dtype=np.float64)}, id_axis=0)
     if cx.rank == 0:
         per = [len(shard_jobs(folds, S, r, cx.world)) for r in range(cx.world)]
         dt = float(np.mean(times))
@@ -840,21 +879,28 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-api-e2e", action="store_true",
                     help="N = 1: skip the fit + predict + score through the public MMSBM API")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
     shape = WORKLOADS[args.workload]
-    if args.impl == "reference":
-        run_reference_arm(args, shape)
-        return
-    cx = Ctx()
-    try:
-        if args.workload == "ml1m_cv":
-            run_cv(args, shape, cx)
-        elif cx.world == 1:
-            run_single(args, shape, cx)
-        else:
-            run_multi(args, shape, cx)
-    finally:
-        cx.close()
+    if args.dump_outputs:
+        args.dump_outputs = os.path.abspath(args.dump_outputs)
+        if args.impl == "reference" or (int(os.environ.get("WORLD_SIZE", "1")) > 1 and args.workload != "ml1m_cv"):
+            raise SystemExit("bench.py: --dump-outputs is supported for --impl b200 on one GPU and for ml1m_cv")
+    with tempfile.TemporaryDirectory(prefix="mmsbm_bench_") as work, contextlib.chdir(work):
+        if args.impl == "reference":
+            run_reference_arm(args, shape)
+            return
+        cx = Ctx()
+        try:
+            if args.workload == "ml1m_cv":
+                run_cv(args, shape, cx)
+            elif cx.world == 1:
+                run_single(args, shape, cx)
+            else:
+                run_multi(args, shape, cx)
+        finally:
+            cx.close()
 
 
 if __name__ == "__main__":

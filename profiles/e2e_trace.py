@@ -1,5 +1,5 @@
-import sys, time, numpy as np, torch
-sys.path.insert(0, "/root/repo")
+import os, sys, time, numpy as np, torch
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
 from mmsbm_b200 import _lib
 U, I, N, K, L, S = bench.WORKLOADS["ml20m"]; R = 5

@@ -97,8 +97,6 @@ def test_bad_ids_raise(kb):
 def test_index_build_bit_exact(shape, heavy):
     from mmsbm_b200.engine import Engine
     N, U, I, R = shape
-    if heavy and N < 1000:
-        pytest.skip("tiny")
     data = random_triples(17, N, U, I, R, heavy_tail=heavy)
     e = Engine(data, U, I, R, 2, 2)
     for col, seg, adj, perm, deg, n_ids in ((0, e.useg, e.uadj, e.uperm, e.udeg, U),
@@ -250,7 +248,7 @@ def test_debug_mode_and_dropped_test_rows(tmp_path, monkeypatch, caplog):
     mm.fit(mock_data(1), silent=True)
     assert len(mm.results) == 2 and all(np.isfinite(r["likelihood"]) for r in mm.results)
     test = pd.concat([mock_data(2, n=20), pd.DataFrame({"users": ["ghost"], "items": ["item1"], "ratings": [3]})])
-    logging.getLogger("MMSBM").propagate = True
+    monkeypatch.setattr(logging.getLogger("MMSBM"), "propagate", True)
     with caplog.at_level(logging.WARNING, logger="MMSBM"):
         pred = mm.predict(test)
     assert pred.shape == (20, 5)
