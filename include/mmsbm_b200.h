@@ -158,6 +158,20 @@ int mmsbm_em_run(const int32_t* useg_dev, const int32_t* uadj_dev, const int32_t
 int mmsbm_em_finalize(double* eta_dev, const int32_t* ideg_dev, int32_t n_items, int32_t L,
                       double* pr_dev, int32_t K, int32_t n_levels, int32_t n_runs, void* stream);
 
+/* ---- fold-in: parameters for ids the fitted model has not seen, with everything else fixed.
+ *      EM on the rows of the new ids alone (the theta or eta update of mmsbm_em_step restricted to
+ *      them); side 0 = new users (own = theta rows, other = eta [S][n_other][ldl]), side 1 = new items
+ *      (own = eta rows, other = theta [S][n_other][ldk]).  seg/adj/deg: the index of the new rows from
+ *      mmsbm_graph_build_side, new ids shifted to 0..n_new-1, neighbour ids global (< n_other).
+ *      own_dev [S][n_new][ld] holds the initial rows on entry and the rows after ``iterations``
+ *      steps on return.  Asynchronous on ``stream``; see csrc/fold_in.cu. */
+int mmsbm_fold_in_workspace_bytes(int64_t n_ratings, int32_t side, int32_t n_new, int32_t n_other,
+                                  int32_t n_levels, int32_t K, int32_t L, int32_t n_runs, size_t* bytes);
+int mmsbm_fold_in(const int32_t* seg_dev, const int32_t* adj_dev, const int32_t* deg_dev, int64_t n_ratings,
+                  int32_t side, int32_t n_new, int32_t n_other, int32_t n_levels, int32_t K, int32_t L,
+                  int32_t n_runs, int32_t iterations, const double* other_dev, const double* pr_dev,
+                  double* own_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
 /* ---- a9 / e3: ONE set of S runs sharded over the GPUs of a box, one process per GPU; replaces the
  *      process pool of src/mmsbm.py:182-185 for a fit too slow or too large for one GPU.
  *      Rank g owns a contiguous user range and a contiguous item range (both balanced by rating

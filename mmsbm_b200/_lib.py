@@ -57,6 +57,8 @@ _PROTOS = {
     "mmsbm_em_step": (C.c_int, [_vp] * 8 + [_i64] + [_i32] * 6 + [_vp] * 6 + [_i32, _vp, _sz, _vp]),
     "mmsbm_em_step_profiled": (C.c_int, [_vp] * 8 + [_i64] + [_i32] * 6 + [_vp] * 6 + [_i32, _vp, _sz, _vp, _vp]),
     "mmsbm_em_run": (C.c_int, [_vp] * 8 + [_i64] + [_i32] * 7 + [_vp] * 6 + [_vp, _sz, _vp]),
+    "mmsbm_fold_in_workspace_bytes": (C.c_int, [_i64] + [_i32] * 7 + [C.POINTER(_sz)]),
+    "mmsbm_fold_in": (C.c_int, [_vp] * 3 + [_i64] + [_i32] * 8 + [_vp] * 3 + [_vp, _sz, _vp]),
     "mmsbm_em_finalize": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _i32, _i32, _i32, _vp]),
     "mmsbm_likelihood_workspace_bytes": (C.c_int, [_i64] + [_i32] * 6 + [C.POINTER(_sz)]),
     "mmsbm_likelihood_min_workspace_bytes": (C.c_int, [_i64] + [_i32] * 6 + [C.POINTER(_sz)]),

@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libmmsbm_b200.so")
 SOURCES = ["em_step.cu", "em_small.cu", "seg_inst_ch1.cu", "seg_inst_ch2.cu", "seg_inst_ch4.cu", "seg_inst_pair.cu", "seg_inst_hexa.cu", "graph_build.cu",
-           "reductions.cu", "host_api.cu", "sharded_run.cu"]
+           "reductions.cu", "host_api.cu", "sharded_run.cu", "fold_in.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
     "-Xcompiler", "-fPIC,-O3,-Wall", "-DMMSBM_B200",   # no --use_fast_math: IEEE fp64 throughout

@@ -208,5 +208,67 @@ class DataHandler:
             enc[:, c] = lut[codes] if len(codes) else 0
         return enc[alive]
 
+    def plan_fold_in(self, data):
+        """Host side of ``MMSBM.fold_in``: encode the rows of ``data`` (read by position, cells
+        ``str()``-ed) against the fitted dictionaries and split them into the two fold-in sets.
+        Nothing is changed; ``add_fold_in_ids`` records the new ids once they have parameters.
+
+        Rows with a rating value unseen in training, and rows whose user and item are both new, are
+        dropped; rows whose user and item are both known are ignored; each with a warning.  New
+        users (items) get the codes after the existing ones, ranked among themselves by
+        ``sorted(set(str))``.  Returns {"users", "items": new labels in code order,
+        "user_rows": int [n,3] (new user - first new code, item, rating),
+        "item_rows": int [m,3] (user, new item - first new code, rating)}."""
+        logger = logging.getLogger("MMSBM")
+        if data.shape[1] < 3:
+            raise ValueError("fold-in data needs three columns: users, items, ratings")
+        parts = _distinct_strings_all([data.iloc[:, c] for c in range(3)])
+        codes = []
+        for (col, strings), table in zip(parts, (self.obs_dict, self.items_dict, self.ratings_dict)):
+            lut = np.array([table.get(s, -1) for s in strings], dtype=np.int64)
+            codes.append(lut[col] if len(col) else np.zeros(0, dtype=np.int64))
+        labels = [np.array(strings, dtype=object)[col] if len(col) else np.zeros(0, dtype=object)
+                  for col, strings in parts]
+        cu, ci, cr = codes
+        alive = np.ones(len(cu), dtype=bool)
+
+        def listed(values):
+            return ", ".join(sorted(set(str(a) for a in values)))
+
+        bad_r = cr < 0
+        if bad_r.any():
+            logger.warning(f"The ratings {listed(labels[2][bad_r])} are in the fold-in set but weren't in the "
+                           f"train set so I'll remove them.")
+            alive &= ~bad_r
+        both_new = alive & (cu < 0) & (ci < 0)
+        if both_new.any():
+            logger.warning(f"The users {listed(labels[0][both_new])} are in the fold-in set with items "
+                           f"{listed(labels[1][both_new])} and neither was in the train set so I'll remove "
+                           f"those {int(both_new.sum())} rows.")
+            alive &= ~both_new
+        both_known = alive & (cu >= 0) & (ci >= 0)
+        if both_known.any():
+            logger.warning(f"The users {listed(labels[0][both_known])} and items {listed(labels[1][both_known])} "
+                           f"of {int(both_known.sum())} fold-in rows were in the train set so I'll ignore "
+                           f"those rows: fit again to use them.")
+            alive &= ~both_known
+        out = {}
+        for name, c, table, own, rows_name in (("users", 0, self.obs_dict, cu, "user_rows"),
+                                              ("items", 1, self.items_dict, ci, "item_rows")):
+            sel = alive & (own < 0)
+            new = sorted(set(labels[c][sel].tolist()))
+            rank = {s: k for k, s in enumerate(new)}
+            rows = np.stack([cu[sel], ci[sel], cr[sel]], axis=1).astype(np.int64).reshape(-1, 3)
+            rows[:, c] = [rank[s] for s in labels[c][sel].tolist()]
+            out[name], out[rows_name] = new, rows
+        return out
+
+    def add_fold_in_ids(self, users, items):
+        """Give the labels of ``plan_fold_in`` their codes after the existing ones."""
+        for table, new in ((self.obs_dict, users), (self.items_dict, items)):
+            base = len(table)
+            for k, s in enumerate(new):
+                table[s] = base + k
+
     def return_dicts(self):
         return self.obs_dict, self.items_dict, self.ratings_dict

@@ -191,6 +191,82 @@ class Engine:
     def swap(self):
         (self.theta, self.eta, self.pr), self._alt = self._alt, (self.theta, self.eta, self.pr)
 
+    # ------------------------------------------------------------------- fold-in
+    def fold_in(self, side, rows, init, iterations):
+        """Rows for ids the engine has not seen, with the parameters it holds fixed.
+
+        ``side`` 0: new users, ``rows`` int [n,3] (user, item, rating) with the new users numbered
+        0..n_new-1 and known item ids; ``init`` [S,n_new,K].  ``side`` 1: new items, mirror case,
+        ``init`` [S,n_new,L].  Runs ``iterations`` EM steps of the new rows alone (csrc/fold_in.cu)
+        and returns them as numpy [S,n_new,K or L]; the engine's parameters are not changed."""
+        if side not in (0, 1):
+            raise ValueError("side must be 0 (users) or 1 (items)")
+        if self.theta is None:
+            raise RuntimeError("the engine holds no parameters: set_params first")
+        rows, init = np.asarray(rows), np.asarray(init, dtype=np.float64)
+        width, ld = (self.K, self.ldk) if side == 0 else (self.L, self.ldl)
+        if rows.ndim != 2 or rows.shape[1] != 3:
+            raise ValueError("rows must have shape [N,3]")
+        if init.ndim != 3 or init.shape[0] != self.S or init.shape[1] < 1 or init.shape[2] != width:
+            raise ValueError(f"init must have shape [{self.S}, n_new, {width}]")
+        n_new, n = int(init.shape[1]), int(rows.shape[0])
+        n_other = self.I if side == 0 else self.U
+        i32 = torch.int32
+        with torch.cuda.device(self.device):
+            raw = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.int64)).to(self.device)
+            cols = torch.empty((3, max(n, 1)), dtype=i32, device=self.device)
+            bad = torch.zeros(1, dtype=i32, device=self.device)
+            nu, ni = (n_new, self.I) if side == 0 else (self.U, n_new)
+            _lib.check(self.lib.mmsbm_split_triples(
+                raw.data_ptr(), n, nu, ni, self.R, cols[0].data_ptr(), cols[1].data_ptr(), cols[2].data_ptr(),
+                bad.data_ptr(), self._stream()), "split_triples")
+            if int(bad.item()):
+                raise ValueError("rows hold an id outside the new ids, the known ids or the rating levels")
+            seg, adj, perm, deg = (self._empty(n_new * self.R + 1, i32), self._empty(n, i32),
+                                   self._empty(n, i32), self._empty(n_new, i32))
+            n_sched = _lib.C.c_int64(0)
+            _lib.check(self.lib.mmsbm_sched_elems(n, n_new, _lib.C.byref(n_sched)), "sched_elems")
+            sched = self._empty(n_sched.value, i32)
+            need = _lib.C.c_size_t(0)
+            _lib.check(self.lib.mmsbm_graph_workspace_bytes(n, n_new, n_new, self.R, _lib.C.byref(need)),
+                       "graph_workspace_bytes")
+            gws = self._bytes(need.value)
+            _lib.check(self.lib.mmsbm_graph_build_side(
+                cols[side].data_ptr(), cols[1 - side].data_ptr(), cols[2].data_ptr(), n, n_new, self.R,
+                seg.data_ptr(), adj.data_ptr(), perm.data_ptr(), deg.data_ptr(), sched.data_ptr(),
+                gws.data_ptr(), need.value, self._stream()), "graph_build_side")
+            own = torch.from_numpy(self._pad(init, ld)).to(self.device)
+            _lib.check(self.lib.mmsbm_fold_in_workspace_bytes(n, side, n_new, n_other, self.R, self.K, self.L,
+                                                              self.S, _lib.C.byref(need)),
+                       "fold_in_workspace_bytes")
+            ws = self._bytes(need.value)
+            _lib.check(self.lib.mmsbm_fold_in(
+                seg.data_ptr(), adj.data_ptr(), deg.data_ptr(), n, side, n_new, n_other, self.R, self.K, self.L,
+                self.S, int(iterations), (self.eta if side == 0 else self.theta).data_ptr(), self.pr.data_ptr(),
+                own.data_ptr(), ws.data_ptr(), need.value, self._stream()), "fold_in")
+            return np.ascontiguousarray(own.cpu().numpy()[..., :width])
+
+    def append_rows(self, side, rows):
+        """Append ``rows`` [S,n,K] to theta (side 0) or [S,n,L] to eta (side 1) of every run, on the
+        device; the new ids follow the existing ones.  The index structure of the training rows
+        does not cover them, so the engine becomes parameters-only (like ``for_prediction``):
+        ``predict`` serves every id, ``run`` / ``likelihood`` need a new fit."""
+        rows = np.asarray(rows, dtype=np.float64)
+        width, ld, cur = (self.K, self.ldk, self.theta) if side == 0 else (self.L, self.ldl, self.eta)
+        if rows.ndim != 3 or rows.shape[0] != self.S or rows.shape[2] != width:
+            raise ValueError(f"rows must have shape [{self.S}, n, {width}]")
+        if rows.shape[1] == 0:
+            return
+        new = torch.cat([cur, torch.from_numpy(self._pad(rows, ld)).to(self.device)], dim=1)
+        if side == 0:
+            self.theta, self.U = new, self.U + rows.shape[1]
+        else:
+            self.eta, self.I = new, self.I + rows.shape[1]
+        self._alt = (torch.empty_like(self.theta), torch.empty_like(self.eta), torch.empty_like(self.pr))
+        self.useg = self.uadj = self.uperm = self.udeg = self.usched = None
+        self.iseg = self.iadj = self.iperm = self.ideg = self.isched = None
+        self._ws, self._ws_bytes = None, 0
+
     # ---------------------------------------------------------------- reductions
     def likelihood_device(self):
         self._need_ratings()

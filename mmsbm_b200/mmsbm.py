@@ -158,17 +158,20 @@ class MMSBM:
             self._index_cache = out
         return self._index_cache
 
+    def _has_index(self):
+        return self._engine is not None and self._engine.useg is not None
+
     @property
     def _user_indices(self):
-        return None if self._engine is None else self._index_lists()["user"]
+        return self._index_lists()["user"] if self._has_index() else None
 
     @property
     def _item_indices(self):
-        return None if self._engine is None else self._index_lists()["item"]
+        return self._index_lists()["item"] if self._has_index() else None
 
     @property
     def _rating_indices(self):
-        return None if self._engine is None else self._index_lists()["rating"]
+        return self._index_lists()["rating"] if self._has_index() else None
 
     def _initial_parameters(self, seed):
         """theta0, eta0, pr0 of one run: three draws in this order from
@@ -321,6 +324,57 @@ class MMSBM:
                 f"The final accuracy is {stats['accuracy']}, the one off accuracy is {stats['one_off_accuracy']} "
                 f"and the MAE is {stats['mae']}.")
         return {"stats": stats, "objects": {"theta": self.theta, "eta": self.eta, "pr": self.pr}}
+
+    # ---------------------------------------------------------------------- fold_in
+    def fold_in(self, data, iterations=None, seed=0):
+        """Parameters for users and items the fitted model has not seen, without refitting.
+
+        ``data``: a DataFrame read by position like ``fit``.  A row of a new user with a known item
+        is used for that user's theta, a row of a known user with a new item for that item's eta;
+        the rest is dropped or ignored with a warning (DataHandler.plan_fold_in).  With eta and pr
+        (theta and pr) fixed, ``iterations`` (default: ``self.iterations``) EM steps run on the new
+        rows alone, for every run; the known rows of every run stay as they are.  Run s starts from
+        ``default_rng(SeedSequence(seed).spawn(S)[s])``: ``random((new users, K))`` then
+        ``random((new items, L))``, each row divided by max(its fold-in rows, 1).  ``self.rng`` is
+        not used.  Afterwards ``predict`` / ``score`` / ``save`` serve the new ids.
+
+        Returns {"users": [...], "items": [...]}: the labels added, in code order."""
+        self._check_is_fitted()
+        iterations = self.iterations if iterations is None else int(iterations)
+        plan = self.data_handler.plan_fold_in(data)
+        added = {"users": plan["users"], "items": plan["items"]}
+        nu, ni = len(plan["users"]), len(plan["items"])
+        if not nu and not ni:
+            return added
+        S, K, L = len(self.results), self.user_groups, self.item_groups
+        engine = self._engine
+        if engine is None:                                    # rating-sharded fit: parameters only
+            engine = self._engine = Engine.for_prediction(self.p + 1, self.m + 1, self._dims['n_ratings'],
+                                                          K, L)
+        if self._resident != list(range(S)) or engine.S != S:
+            engine.set_params(np.array([a["theta"] for a in self.results]),
+                              np.array([a["eta"] for a in self.results]),
+                              np.array([a["pr"] for a in self.results]))
+            self._resident = list(range(S))
+        du = np.maximum(np.bincount(plan["user_rows"][:, 0], minlength=nu), 1)[:, None]
+        di = np.maximum(np.bincount(plan["item_rows"][:, 1], minlength=ni), 1)[:, None]
+        init_u, init_i = np.empty((S, nu, K)), np.empty((S, ni, L))
+        for s, child in enumerate(np.random.SeedSequence(seed).spawn(S)):
+            rng = np.random.default_rng(child)
+            init_u[s] = rng.random((nu, K)) / du
+            init_i[s] = rng.random((ni, L)) / di
+        # both sets are computed from the known rows only, so neither depends on the other
+        new_theta = engine.fold_in(0, plan["user_rows"], init_u, iterations) if nu else init_u
+        new_eta = engine.fold_in(1, plan["item_rows"], init_i, iterations) if ni else init_i
+        engine.append_rows(0, new_theta)
+        engine.append_rows(1, new_eta)
+        for s, res in enumerate(self.results):
+            res["theta"] = np.concatenate([res["theta"], new_theta[s]])
+            res["eta"] = np.concatenate([res["eta"], new_eta[s]])
+        self.data_handler.add_fold_in_ids(plan["users"], plan["items"])
+        self.p, self.m = self.p + nu, self.m + ni
+        self._index_cache = None
+        return added
 
     # ----------------------------------------------------------------------- cv_fit
     def _make_folds(self, data, folds):
