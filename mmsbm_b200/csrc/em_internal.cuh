@@ -15,9 +15,12 @@ void set_reserved_ctas(int n);
 
 // How the S runs of a launch row are served by the segment pass for neighbour rows of NBp
 // doubles: runs [0, 6*hexas) six per warp, then `pairs` pairs (pair groups numbered over ALL
-// runs, first one = pair_group0), the rest one run per warp from run `single_from`.
+// runs, first one = pair_group0), the rest one run per warp from run `single_from`.  A group
+// of runs is planned only when its w rows (R levels) fit the shared memory of a CTA: six runs
+// fall back to pairs, pairs to one run per warp.  The tables of interleaved rows are filled for
+// exactly the planned groups.
 struct RunPlan { int hexas, pairs, pair_group0, single_from; };
-RunPlan plan_runs(int NBp, int n_runs, bool hexa_table);
+RunPlan plan_runs(int NBp, int R, int n_runs, bool hexa_table);
 
 int launch_prep_p(const double* pr, int K, int L, int R, int ldk, int ldl, int n_runs, double* pw_u,
                   double* pn_u, double* pw_i, double* pn_i, cudaStream_t st);
@@ -30,7 +33,8 @@ int launch_interleave(const double* src, double* dst, int n_src, int n_dst, int 
 
 int launch_w(const double* own, const double* pw, double* W, int M, int LD, int RNB, int n_runs,
              cudaStream_t st);
-// Where row_n_kernel ALSO writes the new rows, in the run-interleaved layout of a gather table that
+// Where launch_n ALSO writes the new rows (row_n_kernel stores them itself, the tiled path copies them
+// afterwards), in the run-interleaved layout of a gather table that
 // spans all ranks (a sharded run publishes its new rows this way instead of re-reading them with
 // interleave_runs_kernel): table t serves the runs [gs*group0, gs*(group0+groups)) and holds
 // dst[((run/gs) * n_all + row0 + row) * gs + run%gs][ld].

@@ -45,7 +45,7 @@ namespace mmsbm {
 constexpr int kPrThreads = 128;
 constexpr int kPrBatch = 16;    // segments staged per smem batch
 constexpr int kGemmThreads = 256;
-constexpr int kGemmBK = 32;     // k-slab of the small GEMM (even)
+constexpr int kGemmBK = 32;     // k-slab of the small GEMM (lower when a streamed slab of B does not fit)
 constexpr int kGemmTR = 4;      // rows per thread tile of the small GEMM
 
 // g rows of long segments: add the partial rows of their pieces in piece order
@@ -108,8 +108,10 @@ __global__ void prep_p_kernel(const double* pr, int K, int L, int R, int ldk, in
 
 // ---- C[M x N] = A[M x Kd] . B[Kd x N] for tall-skinny fp64 problems (N, Kd <= ~1k) ------------
 // Persistent CTAs: B is staged in shared memory once, then each CTA walks row tiles; one 4x4
-// output tile per thread (rg row groups x N/4 column groups), A in k-slabs of kGemmBK.  EPI: C = C o own / max(deg,1).  fp64 FMA pipe, no tensor
-// cores (B200 DMMA is no faster than the vector pipe and the path is not GEMM-bound).
+// output tile per thread (rg row groups x N/4 column groups), A in k-slabs of g.bk rows (B too, when
+// it does not fit shared memory whole).  Every thread adds its products in increasing k whatever
+// the slab height, so the height does not change the result.  EPI: C = C o own / max(deg,1).
+// fp64 FMA pipe, no tensor cores (B200 DMMA is no faster than the vector pipe and the path is not GEMM-bound).
 struct GemmArgs {
   const double* A;      // [S][M][lda]
   const double* B;      // [S][Kd][N]
@@ -118,15 +120,16 @@ struct GemmArgs {
   const int32_t* deg;   // EPI: [M]
   int M, N, Kd, lda, rg, normalize;
   int b_resident;       // whole B staged once (fits shared memory) or one k-slab at a time
+  int bk;               // k-slab height: a multiple of 4, kGemmBK unless a slab of B would not fit
 };
 
 template <bool EPI>
 __global__ void __launch_bounds__(kGemmThreads) small_gemm_kernel(const GemmArgs g) {
   constexpr int TR = kGemmTR;                  // rows of the register tile (columns: 4)
   extern __shared__ __align__(32) unsigned char smem_raw[];
-  const int BM = TR * g.rg, AS = kGemmBK + 2;
-  double* Bs = reinterpret_cast<double*>(smem_raw);          // [Kd][N] whole B, or [kGemmBK][N] slab
-  double* As = Bs + (size_t)(g.b_resident ? g.Kd : kGemmBK) * g.N;   // [BM][AS] k-slab of a row tile
+  const int BM = TR * g.rg, AS = g.bk + 2;
+  double* Bs = reinterpret_cast<double*>(smem_raw);          // [Kd][N] whole B, or [bk][N] slab
+  double* As = Bs + (size_t)(g.b_resident ? g.Kd : g.bk) * g.N;   // [BM][AS] k-slab of a row tile
   const int run = blockIdx.y;
   const int ncg = g.N >> 2, half = g.N >> 1;
   const int rgid = threadIdx.x / ncg, cg = threadIdx.x - rgid * ncg;
@@ -145,8 +148,8 @@ __global__ void __launch_bounds__(kGemmThreads) small_gemm_kernel(const GemmArgs
 #pragma unroll
       for (int j = 0; j < 4; ++j) acc[i][j] = 0.0;
 
-    for (int k0 = 0; k0 < g.Kd; k0 += kGemmBK) {
-      const int bk = min(kGemmBK, g.Kd - k0);          // multiple of 4
+    for (int k0 = 0; k0 < g.Kd; k0 += g.bk) {
+      const int bk = min(g.bk, g.Kd - k0);             // multiple of 4
       const int bk2 = bk >> 1;
       __syncthreads();
       for (int t = threadIdx.x; t < BM * bk2; t += kGemmThreads) {   // 128-bit staging of the A slab
@@ -546,9 +549,10 @@ static int segs_per_cta_for(int64_t pmax, int64_t n_ratings, int grid_y) {
   return (int)spc;
 }
 
-// pairs of runs per warp whenever there are at least two runs and a lane holds one chunk
-static bool pairs_enabled(int NBp, int n_runs) {
-  return n_runs >= 2 && NBp <= 32 && env_int("MMSBM_PAIR", 1) != 0;
+// pairs of runs per warp whenever there are at least two runs, a lane holds one chunk and the
+// w rows of a pair fit shared memory
+static bool pairs_enabled(int NBp, int R, int n_runs) {
+  return n_runs >= 2 && NBp <= 32 && seg_smem_bytes(R, NBp, 2) <= kMaxSmemBytes && env_int("MMSBM_PAIR", 1) != 0;
 }
 
 // grid.x of a segment pass.  The piece count lives on the device, so the grid is sized for its upper
@@ -565,16 +569,17 @@ static unsigned grid_x_for(const SegArgs& a, int ctas_per_sm) {
   return (unsigned)(want < resident ? want : resident);
 }
 
-// six runs per warp: rows of exactly 20 doubles (5-lane groups, 30 of 32 lanes), at least six runs
-static bool hexa_enabled(int NBp, int n_runs) {
-  return n_runs >= 6 && NBp == 20 && env_int("MMSBM_HEXA", 1) != 0;
+// six runs per warp: rows of exactly 20 doubles (5-lane groups, 30 of 32 lanes), at least six runs,
+// and the w rows of six runs fit shared memory (R <= 30)
+static bool hexa_enabled(int NBp, int R, int n_runs) {
+  return n_runs >= 6 && NBp == 20 && seg_smem_bytes(R, NBp, 6) <= kMaxSmemBytes && env_int("MMSBM_HEXA", 1) != 0;
 }
 
-RunPlan plan_runs(int NBp, int n_runs, bool hexa_table) {
+RunPlan plan_runs(int NBp, int R, int n_runs, bool hexa_table) {
   RunPlan p{0, 0, 0, 0};
-  if (hexa_table && hexa_enabled(NBp, n_runs)) p.hexas = n_runs / 6;
+  if (hexa_table && hexa_enabled(NBp, R, n_runs)) p.hexas = n_runs / 6;
   p.single_from = 6 * p.hexas;
-  if (pairs_enabled(NBp, n_runs - p.single_from)) {
+  if (pairs_enabled(NBp, R, n_runs - p.single_from)) {
     p.pairs = (n_runs - p.single_from) / 2;
     p.pair_group0 = p.single_from / 2;            // pairs are numbered over all runs (6 | single_from)
     p.single_from += 2 * p.pairs;
@@ -587,7 +592,7 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
   const double avg_degree = (double)n_ratings / (double)a.nseg;
   PassShape sh = choose_shape(a.NBp, avg_degree);
   const int un_e = env_int("MMSBM_UN", 0), occ_e = env_int("MMSBM_OCC", 0);
-  const RunPlan plan = plan_runs(a.NBp, n_runs, nbr_hexa != nullptr);
+  const RunPlan plan = plan_runs(a.NBp, a.R, n_runs, nbr_hexa != nullptr);
   const int single_from = plan.single_from;      // runs [single_from, n_runs) go one run per warp
   if (plan.hexas > 0) {
     const int hexas = plan.hexas;
@@ -598,8 +603,7 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
     p.segs_per_cta = segs_per_cta_for(a.pmax, n_ratings, hexas);
     const unsigned gx = grid_x_for(p, occ_e > 0 ? occ_e : 3);
     if (p.counters) a.counters += hexas;         // the next launch of this pass gets its own counters
-    const size_t smem = seg_smem_bytes(p, 6);
-    MMSBM_REQUIRE(smem <= 227 * 1024, MMSBM_ERANGE, "segment pass needs %zu bytes of shared memory", smem);
+    const size_t smem = seg_smem_bytes(a.R, a.NBp, 6);   // fits: plan_runs checked it
     int rc = MMSBM_ERANGE;
     if (un_e > 0 || occ_e > 0)
       rc = launch_segment_pass_hexa(p, sh.G, un_e > 0 ? un_e : 3, occ_e > 0 ? occ_e : 3, dim3(gx, hexas), smem, st);
@@ -621,8 +625,7 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
     p.segs_per_cta = segs_per_cta_for(a.pmax, n_ratings, pairs);
     const unsigned gx = grid_x_for(p, occ_e > 0 ? occ_e : 3);
     if (p.counters) a.counters += pairs;
-    const size_t smem = seg_smem_bytes(p, 2);
-    MMSBM_REQUIRE(smem <= 227 * 1024, MMSBM_ERANGE, "segment pass needs %zu bytes of shared memory", smem);
+    const size_t smem = seg_smem_bytes(a.R, a.NBp, 2);   // fits: plan_runs checked it
     int UN = (sh.G == 1) ? 2 : 3, MINB = 3;                     // UN * (32 / 2G) <= 32
     int rc = MMSBM_ERANGE;
     if (un_e > 0 || occ_e > 0)
@@ -639,8 +642,8 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
   a.segs_per_cta = segs_per_cta_for(a.pmax, n_ratings, n_runs - single_from);
   const unsigned gx = grid_x_for(a, occ_e > 0 ? occ_e : sh.MINB);
   const dim3 grid(gx, n_runs - single_from);
-  const size_t smem = seg_smem_bytes(a, 1);
-  MMSBM_REQUIRE(smem <= 227 * 1024, MMSBM_ERANGE,
+  const size_t smem = seg_smem_bytes(a.R, a.NBp, 1);
+  MMSBM_REQUIRE(smem <= kMaxSmemBytes, MMSBM_ERANGE,
                 "segment pass needs %zu bytes of shared memory (R=%d, row stride %d)", smem, a.R, a.NBp);
   auto go = [&](const PassShape& p) {
     switch (p.CH) {
@@ -684,10 +687,16 @@ static int launch_gemm(GemmArgs g, int n_runs, cudaStream_t st) {
   if (rg > 32) rg = 32;
   g.rg = rg;
   const int BM = kGemmTR * rg;
-  size_t smem = ((size_t)g.Kd * g.N + (size_t)BM * (kGemmBK + 2)) * 8;
+  g.bk = kGemmBK;
+  size_t smem = ((size_t)g.Kd * g.N + (size_t)BM * (g.bk + 2)) * 8;
   g.b_resident = smem <= 200 * 1024;
-  if (!g.b_resident) smem = ((size_t)kGemmBK * g.N + (size_t)BM * (kGemmBK + 2)) * 8;
-  MMSBM_REQUIRE(smem <= 227 * 1024, MMSBM_ERANGE,
+  if (!g.b_resident) {
+    // streamed B: slabs of kGemmBK rows where they fit, otherwise the tallest multiple of 4 that does
+    auto slab_bytes = [&](int bk) { return ((size_t)bk * g.N + (size_t)BM * (bk + 2)) * 8; };
+    while (g.bk > 4 && slab_bytes(g.bk) > kMaxSmemBytes) g.bk -= 4;
+    smem = slab_bytes(g.bk);
+  }
+  MMSBM_REQUIRE(smem <= kMaxSmemBytes, MMSBM_ERANGE,
                 "small gemm needs %zu bytes of shared memory (K*L*R too large)", smem);
   auto kern = small_gemm_kernel<EPI>;
   MMSBM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -720,7 +729,7 @@ int launch_w(const double* own, const double* pw, double* W, int M, int LD, int 
   MMSBM_ROW_W(4) MMSBM_ROW_W(8) MMSBM_ROW_W(12) MMSBM_ROW_W(16) MMSBM_ROW_W(20) MMSBM_ROW_W(24)
   MMSBM_ROW_W(28) MMSBM_ROW_W(32)
 #undef MMSBM_ROW_W
-  GemmArgs g{own, pw, W, nullptr, nullptr, M, RNB, LD, LD, 0, 0, 0};
+  GemmArgs g{own, pw, W, nullptr, nullptr, M, RNB, LD, LD, 0, 0, 0, kGemmBK};
   return launch_gemm<false>(g, n_runs, st);
 }
 
@@ -757,9 +766,16 @@ int launch_n(const double* G, const double* pn, const double* own, const int32_t
   MMSBM_ROW_N(28) MMSBM_ROW_N(32)
 #undef MMSBM_ROW_N_GO
 #undef MMSBM_ROW_N
-  MMSBM_REQUIRE(!publish, MMSBM_ERANGE, "row publishing needs row strides of at most 32 doubles");
-  GemmArgs g{G, pn, out, own, deg, M, LD, RNB, RNB, 0, normalize, 0};
-  return launch_gemm<true>(g, n_runs, st);
+  GemmArgs g{G, pn, out, own, deg, M, LD, RNB, RNB, 0, normalize, 0, kGemmBK};
+  int rc = launch_gemm<true>(g, n_runs, st);
+  if (rc || !publish) return rc;
+  // the tiled path (a P table of more than 200 KB) writes `out` only: copy the new rows into the
+  // gather tables afterwards
+  for (int t = 0; t < 3; ++t)
+    if (pub.dst[t] && (rc = launch_interleave(out, pub.dst[t], M, pub.n_all, pub.row0, LD, pub.group0[t],
+                                              pub.groups[t], pub.gs[t], st)))
+      return rc;
+  return 0;
 }
 
 int launch_prep_p(const double* pr, int K, int L, int R, int ldk, int ldl, int n_runs, double* pw_u,
@@ -897,6 +913,8 @@ static int em_step_impl(const int32_t* useg, const int32_t* uadj, const int32_t*
                 "mmsbm_em_step: K, L <= 256 and R <= 31 supported (K=%d L=%d R=%d)", K, L, R);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   EmDims d = em_dims(N, U, I, R, K, L, S);
+  // run groups of the two segment passes: their interleaved tables are filled below
+  const RunPlan plan_u = plan_runs(d.ldl, R, S, true), plan_i = plan_runs(d.ldk, R, S, false);
   Arena arena(ws, ws_bytes);
   double* pw_u = arena.take<double>(d.p_elems);
   double* pn_u = arena.take<double>(d.p_elems);
@@ -938,8 +956,8 @@ static int em_step_impl(const int32_t* useg, const int32_t* uadj, const int32_t*
                        (flags & MMSBM_RAW_ETA_PR) == 0, s);
     };
     // user branch (main stream)
-    if (hexa_enabled(d.ldl, S) && (rc = launch_interleave(eta, et6, I, I, 0, d.ldl, 0, S / 6, 6, st))) return rc;
-    if (pairs_enabled(d.ldl, S) && (rc = launch_interleave(eta, et2, I, I, 0, d.ldl, 0, S / 2, 2, st))) return rc;
+    if ((rc = launch_interleave(eta, et6, I, I, 0, d.ldl, 0, plan_u.hexas, 6, st))) return rc;
+    if ((rc = launch_interleave(eta, et2, I, I, 0, d.ldl, plan_u.pair_group0, plan_u.pairs, 2, st))) return rc;
     if ((rc = launch_w(theta, pw_u, wg_u, U, d.ldk, d.rnb_u, S, st))) return rc;
     {
       SegArgs a{useg, uadj, usched, eta, wg_u, slots_u, d.pmax_u, d.lmax, d.smax, U, I, d.ldl, R, 0, 0, 0,
@@ -950,7 +968,7 @@ static int em_step_impl(const int32_t* useg, const int32_t* uadj, const int32_t*
                        (flags & MMSBM_RAW_THETA) ? 0 : 1, S, st))) return rc;
     if (!d.emit_items && (rc = pr_step(st))) return rc;
     // item branch (side stream)
-    if (pairs_enabled(d.ldk, S) && (rc = launch_interleave(theta, th2, U, U, 0, d.ldk, 0, S / 2, 2, s2))) return rc;
+    if ((rc = launch_interleave(theta, th2, U, U, 0, d.ldk, plan_i.pair_group0, plan_i.pairs, 2, s2))) return rc;
     if ((rc = launch_w(eta, pw_i, wg_i, I, d.ldl, d.rnb_i, S, s2))) return rc;
     {
       SegArgs a{iseg, iadj, isched, theta, wg_i, slots_i, d.pmax_i, d.lmax, d.smax, I, U, d.ldk, R, 0, 0, 0,
@@ -970,9 +988,9 @@ static int em_step_impl(const int32_t* useg, const int32_t* uadj, const int32_t*
     MMSBM_FORK(0);                                                  // side: after the P tables
     // rows of run groups side by side: eta for the by-user pass (six runs when rows hold 20
     // doubles, pairs), theta for the by-item pass (pairs)
-    if (hexa_enabled(d.ldl, S) && (rc = launch_interleave(eta, et6, I, I, 0, d.ldl, 0, S / 6, 6, st))) return rc;
-    if (pairs_enabled(d.ldl, S) && (rc = launch_interleave(eta, et2, I, I, 0, d.ldl, 0, S / 2, 2, st))) return rc;
-    if (pairs_enabled(d.ldk, S) && (rc = launch_interleave(theta, th2, U, U, 0, d.ldk, 0, S / 2, 2, st))) return rc;
+    if ((rc = launch_interleave(eta, et6, I, I, 0, d.ldl, 0, plan_u.hexas, 6, st))) return rc;
+    if ((rc = launch_interleave(eta, et2, I, I, 0, d.ldl, plan_u.pair_group0, plan_u.pairs, 2, st))) return rc;
+    if ((rc = launch_interleave(theta, th2, U, U, 0, d.ldk, plan_i.pair_group0, plan_i.pairs, 2, st))) return rc;
     if ((rc = launch_w(theta, pw_u, wg_u, U, d.ldk, d.rnb_u, S, st))) return rc;
     if ((rc = launch_w(eta, pw_i, wg_i, I, d.ldl, d.rnb_i, S, s2))) return rc;
     MMSBM_SIDE_DONE(1);                                             // w of the items ready

@@ -289,17 +289,22 @@ struct ProdArgs {
   int U, I, R, K, L, ldk, ldl;
 };
 
+// SMEM_P: pr staged in shared memory as [R][K][L]; otherwise (tables too large for shared memory)
+// read in place from global memory, where it stays L2-resident.  Same products, same order.
+template <bool SMEM_P>
 __global__ void __launch_bounds__(256) prod_dist_kernel(const ProdArgs A) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   const int K = A.K, L = A.L, R = A.R;
-  double* Pq = reinterpret_cast<double*>(smem_raw);          // [R][K][L]
-  double* th_s = Pq + (size_t)R * K * L;                     // [warps][K]
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarp = blockDim.x >> 5;
   const int run = blockIdx.y;
   const double* prs = A.pr + (size_t)run * K * L * R;
-  for (int t = threadIdx.x; t < K * L * R; t += blockDim.x) {
-    int kl = t / R, r = t - kl * R;
-    Pq[(size_t)r * K * L + kl] = __ldg(prs + t);
+  double* Pq = reinterpret_cast<double*>(smem_raw);          // [R][K][L] (SMEM_P)
+  double* th_s = SMEM_P ? Pq + (size_t)R * K * L : Pq;       // [warps][K]
+  if (SMEM_P) {
+    for (int t = threadIdx.x; t < K * L * R; t += blockDim.x) {
+      int kl = t / R, r = t - kl * R;
+      Pq[(size_t)r * K * L + kl] = __ldg(prs + t);
+    }
   }
   __syncthreads();
   double* th = th_s + warp * K;
@@ -313,13 +318,16 @@ __global__ void __launch_bounds__(256) prod_dist_kernel(const ProdArgs A) {
     __syncwarp();
     const double* erow = eta_run + (size_t)it * A.ldl;
     for (int r = 0; r < R; ++r) {
-      const double* Pr = Pq + (size_t)r * K * L;
+      const double* Pr = SMEM_P ? Pq + (size_t)r * K * L : prs + r;
       double acc = 0.0;
       for (int l0 = 0; l0 < L; l0 += 32) {
         const int l = l0 + lane;
         if (l < L) {
           const double e = __ldg(erow + l);
-          for (int k = 0; k < K; ++k) acc = fma(th[k] * e, Pr[k * L + l], acc);
+          for (int k = 0; k < K; ++k) {
+            const double p = SMEM_P ? Pr[k * L + l] : __ldg(Pr + (size_t)(k * L + l) * R);
+            acc = fma(th[k] * e, p, acc);
+          }
         }
       }
       acc = warp_sum(acc);
@@ -424,7 +432,9 @@ constexpr int kStatBlocks = 296;
 
 using namespace mmsbm;
 
-constexpr size_t kLikTableBytes = 512 * 1024;   // room for [2][R][K][L] per run when spilled to global
+// [2][R][K][L] tables of one run of the element-wise likelihood (global memory when they do not fit
+// shared memory)
+static size_t lik_table_bytes(int R, int K, int L) { return 2 * (size_t)R * K * L * 8; }
 
 static int lik_env_int(const char* name, int dflt) {
   const char* v = getenv(name);
@@ -448,7 +458,7 @@ extern "C" int mmsbm_likelihood_workspace_bytes(int64_t N, int32_t U, int32_t I,
                                                 int32_t L, int32_t S, size_t* bytes) {
   MMSBM_REQUIRE(bytes && N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
                 "mmsbm_likelihood_workspace_bytes: bad argument");
-  const size_t elementwise = align_up((size_t)S * kLikCtas * kLikWarps * 8) + align_up((size_t)S * kLikTableBytes) + 256;
+  const size_t elementwise = align_up((size_t)S * kLikCtas * kLikWarps * 8) + align_up((size_t)S * lik_table_bytes(R, K, L)) + 256;
   size_t fact = 0;
   if (lik_factorised_ok(R, K, L))
     fact = align_up((size_t)S * lik_pmax(N, U) * 8) + (size_t)S * lik_run_bytes(U, I, R, L) + 256;
@@ -461,7 +471,7 @@ extern "C" int mmsbm_likelihood_min_workspace_bytes(int64_t N, int32_t U, int32_
                                                     int32_t L, int32_t S, size_t* bytes) {
   MMSBM_REQUIRE(bytes && N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
                 "mmsbm_likelihood_min_workspace_bytes: bad argument");
-  const size_t elementwise = align_up((size_t)S * kLikCtas * kLikWarps * 8) + align_up((size_t)S * kLikTableBytes) + 256;
+  const size_t elementwise = align_up((size_t)S * kLikCtas * kLikWarps * 8) + align_up((size_t)S * lik_table_bytes(R, K, L)) + 256;
   size_t fact = 0;
   if (lik_factorised_ok(R, K, L))
     fact = align_up((size_t)S * lik_pmax(N, U) * 8) + lik_run_bytes(U, I, R, L) + 256;
@@ -560,9 +570,7 @@ extern "C" int mmsbm_likelihood(const int32_t* useg, const int32_t* uadj, const 
   LikArgs a{useg, uadj, theta, eta, pr, partial, nullptr, U, I, R, K, L, row_stride(K), row_stride(L)};
   size_t smem = (2 * (size_t)R * K * L + 2 * (size_t)kLikWarps * K) * 8;
   if (smem > 200 * 1024) {                       // keep the two tables in global memory (L2 resident)
-    const size_t tb = 2 * (size_t)R * K * L * 8;
-    MMSBM_REQUIRE(tb <= kLikTableBytes, MMSBM_ERANGE, "mmsbm_likelihood: K*L*R = %d too large", K * L * R);
-    a.tables = arena.take<double>((size_t)S * 2 * R * K * L);
+    a.tables = arena.take<double>((size_t)S * lik_table_bytes(R, K, L) / 8);
     MMSBM_REQUIRE(a.tables, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
     const int n = K * L * R;
     lik_tables_kernel<<<dim3((n + 255) / 256, S), 256, 0, st>>>(pr, K, L, R, a.tables);
@@ -588,13 +596,16 @@ extern "C" int mmsbm_prod_dist(const int32_t* user, const int32_t* item, int64_t
   if (M == 0) return 0;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   ProdArgs a{user, item, theta, eta, pr, rat, M, U, I, R, K, L, row_stride(K), row_stride(L)};
-  size_t smem = ((size_t)R * K * L + 8 * (size_t)K) * 8;
-  MMSBM_REQUIRE(smem <= 227 * 1024, MMSBM_ERANGE, "mmsbm_prod_dist: K*L*R too large for shared memory");
-  MMSBM_CUDA(cudaFuncSetAttribute(prod_dist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const size_t th_bytes = 8 * (size_t)K * 8;                 // theta rows of the 8 warps
+  size_t smem = (size_t)R * K * L * 8 + th_bytes;
+  const bool smem_p = smem <= kMaxSmemBytes;
+  if (!smem_p) smem = th_bytes;
+  auto kern = smem_p ? prod_dist_kernel<true> : prod_dist_kernel<false>;
+  MMSBM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int64_t want = (M + 7) / 8;
   const int64_t cap = (int64_t)sm_count() * 8;
   unsigned grid = (unsigned)(want < cap ? want : cap);
-  prod_dist_kernel<<<dim3(grid, S), 256, smem, st>>>(a);
+  kern<<<dim3(grid, S), 256, smem, st>>>(a);
   MMSBM_LAUNCH_CHECK("prod_dist_kernel");
   return 0;
 }

@@ -86,9 +86,10 @@ struct SegArgs {
 // w rows in shared memory: double buffered (next piece's rows land while this piece runs) for
 // one run or a pair per warp, single buffered for wider run groups (6 runs: 77 KB per CTA otherwise)
 __host__ __device__ constexpr int w_buffers(int runs) { return runs > 2 ? 1 : 2; }
-inline size_t seg_smem_bytes(const SegArgs& a, int runs) {
-  return (size_t)kWarps * w_buffers(runs) * runs * a.R * a.NBp * 8 + 32;
+inline size_t seg_smem_bytes(int R, int NBp, int runs) {
+  return (size_t)kWarps * w_buffers(runs) * runs * R * NBp * 8 + 32;
 }
+constexpr size_t kMaxSmemBytes = 227 * 1024;   // dynamic shared memory of one CTA on sm_100a
 
 // Sum of `part` over the G consecutive lanes of a group, delivered to every lane of the group.
 // Power-of-two groups are aligned, so xor shuffles do; otherwise windows of 1, 2, 4 lanes are

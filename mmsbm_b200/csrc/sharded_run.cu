@@ -72,9 +72,9 @@ struct GridLayout {
   size_t half_bytes, total_bytes;
 };
 
-static GridLayout grid_layout(int U, int I, int K, int L, int S) {
+static GridLayout grid_layout(int U, int I, int K, int L, int R, int S) {
   const int ldk = row_stride(K), ldl = row_stride(L);
-  const RunPlan pu = plan_runs(ldl, S, true), pi = plan_runs(ldk, S, false);
+  const RunPlan pu = plan_runs(ldl, R, S, true), pi = plan_runs(ldk, R, S, false);
   GridLayout g{};
   size_t off = 0;
   auto put = [&](Table& t, int gs, int group0, int groups, int ld, int n_all, int addr_groups) {
@@ -338,7 +338,14 @@ extern "C" int mmsbm_ipc_free(void* dev_ptr) {
 extern "C" int mmsbm_shard_exchange_bytes(int32_t U, int32_t I, int32_t K, int32_t L, int32_t S, size_t* bytes) {
   MMSBM_REQUIRE(bytes && U > 0 && I > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
                 "mmsbm_shard_exchange_bytes: bad argument");
-  *bytes = grid_layout(U, I, K, L, S).total_bytes;
+  // the layout follows the run plan, which depends on the number of rating levels through shared
+  // memory: the buffer is sized for the largest layout over every supported level count
+  size_t most = 0;
+  for (int R = 1; R <= 31; ++R) {
+    const size_t b = grid_layout(U, I, K, L, R, S).total_bytes;
+    if (b > most) most = b;
+  }
+  *bytes = most;
   return 0;
 }
 
@@ -361,7 +368,7 @@ extern "C" int mmsbm_shard_publish(const mmsbm_shard_t* sh, const double* theta_
   MMSBM_REQUIRE(theta_own && eta_own && (half == 0 || half == 1), MMSBM_EINVAL, "mmsbm_shard_publish: bad argument");
   if (sh->world > 1 && (rc = nccl_ready())) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const GridLayout g = grid_layout(sh->n_users, sh->n_items, sh->K, sh->L, sh->n_runs);
+  const GridLayout g = grid_layout(sh->n_users, sh->n_items, sh->K, sh->L, sh->n_levels, sh->n_runs);
   Exchange ex;
   if ((rc = ex.open(sh->world))) return rc;
   if (sh->world > 1) {                          // the side stream starts behind everything queued on `st`
@@ -420,7 +427,7 @@ extern "C" int mmsbm_em_run_sharded(const mmsbm_shard_t* shp, int32_t iterations
   const int S = sh.n_runs, R = sh.n_levels, K = sh.K, L = sh.L;
   const int Uo = sh.n_users_own, Io = sh.n_items_own;
   const ShardDims d = shard_dims(sh);
-  const GridLayout g = grid_layout(sh.n_users, sh.n_items, K, L, S);
+  const GridLayout g = grid_layout(sh.n_users, sh.n_items, K, L, R, S);
   Arena arena(ws, ws_bytes);
   double* pw_u = arena.take<double>(d.p_elems);
   double* pn_u = arena.take<double>(d.p_elems);

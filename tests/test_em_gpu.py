@@ -150,7 +150,9 @@ def test_fixture_one_and_ten_iterations(golden_dir):
                                      # the BASELINE.json shapes the kernels specialise on: Netflix
                                      # (K=L=32, one run: 8-lane rows on both sides), ML-1M (K=L=10, eight
                                      # runs: pairs of 3-lane rows), ML-100K (K=L=10, one run)
-                                     (32, 32, 5, 1), (10, 10, 5, 8), (10, 10, 5, 1)])
+                                     (32, 32, 5, 1), (10, 10, 5, 8), (10, 10, 5, 1),
+                                     # rows of 16 and 24 doubles (4- and 6-lane groups, alone and in pairs)
+                                     (16, 16, 7, 2), (24, 22, 6, 3)])
 @pytest.mark.parametrize("heavy", [False, True])
 def test_batched_runs_one_iteration_vs_oracle(K, L, R, S, heavy):
     from mmsbm_b200.engine import Engine

@@ -11,7 +11,9 @@ from tests.util import random_params, random_triples, rel_err
 
 pytestmark = pytest.mark.gpu
 
-SHAPES = [(10, 10, 5, 3), (20, 20, 5, 8), (7, 5, 4, 1), (3, 32, 6, 2), (33, 9, 5, 1), (40, 36, 5, 2)]
+SHAPES = [(10, 10, 5, 3), (20, 20, 5, 8), (7, 5, 4, 1), (3, 32, 6, 2), (33, 9, 5, 1), (40, 36, 5, 2),
+          # whole-warp rows of 4 and 8 doubles per lane (fold_in_kernel<32, 4> and <32, 8>)
+          (100, 5, 10, 2), (256, 3, 4, 1)]
 
 
 def caps(width):
