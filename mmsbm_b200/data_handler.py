@@ -75,6 +75,10 @@ def _rank_table(strings):
     return {s: k for k, s in enumerate(sorted(set(strings.tolist())))}
 
 
+def _listed(values):
+    return ", ".join(sorted(set(str(a) for a in values)))
+
+
 def _encode(strings, table):
     uniq, inv = np.unique(strings.astype(str), return_inverse=True) if len(strings) > 64 \
         else (None, None)
@@ -208,6 +212,34 @@ class DataHandler:
             enc[:, c] = lut[codes] if len(codes) else 0
         return enc[alive]
 
+    def _encode_known(self, data, what):
+        """Rows of ``data`` (read by position, cells ``str()``-ed) encoded against the fitted
+        dictionaries, shared by ``plan_fold_in`` and ``plan_refit``.  Returns (codes, labels, alive):
+        the int code per column (-1 where the value is unknown), the ``str`` label per column, and
+        the rows whose rating value is known (the others are dropped with a warning)."""
+        if data.shape[1] < 3:
+            raise ValueError(f"{what} data needs three columns: users, items, ratings")
+        parts = _distinct_strings_all([data.iloc[:, c] for c in range(3)])
+        codes = []
+        for (col, strings), table in zip(parts, (self.obs_dict, self.items_dict, self.ratings_dict)):
+            lut = np.array([table.get(s, -1) for s in strings], dtype=np.int64)
+            codes.append(lut[col] if len(col) else np.zeros(0, dtype=np.int64))
+        labels = [np.array(strings, dtype=object)[col] if len(col) else np.zeros(0, dtype=object)
+                  for col, strings in parts]
+        alive = codes[2] >= 0
+        if not alive.all():
+            logging.getLogger("MMSBM").warning(
+                f"The ratings {_listed(labels[2][~alive])} are in the {what} set but weren't in the "
+                f"train set so I'll remove them.")
+        return codes, labels, alive
+
+    @staticmethod
+    def _rank_new(labels):
+        """(new labels ranked by ``sorted(set(str))``, the rank of every row's label)."""
+        new = sorted(set(labels.tolist()))
+        rank = {s: k for k, s in enumerate(new)}
+        return new, np.array([rank[s] for s in labels.tolist()], dtype=np.int64)
+
     def plan_fold_in(self, data):
         """Host side of ``MMSBM.fold_in``: encode the rows of ``data`` (read by position, cells
         ``str()``-ed) against the fitted dictionaries and split them into the two fold-in sets.
@@ -220,35 +252,17 @@ class DataHandler:
         "user_rows": int [n,3] (new user - first new code, item, rating),
         "item_rows": int [m,3] (user, new item - first new code, rating)}."""
         logger = logging.getLogger("MMSBM")
-        if data.shape[1] < 3:
-            raise ValueError("fold-in data needs three columns: users, items, ratings")
-        parts = _distinct_strings_all([data.iloc[:, c] for c in range(3)])
-        codes = []
-        for (col, strings), table in zip(parts, (self.obs_dict, self.items_dict, self.ratings_dict)):
-            lut = np.array([table.get(s, -1) for s in strings], dtype=np.int64)
-            codes.append(lut[col] if len(col) else np.zeros(0, dtype=np.int64))
-        labels = [np.array(strings, dtype=object)[col] if len(col) else np.zeros(0, dtype=object)
-                  for col, strings in parts]
+        codes, labels, alive = self._encode_known(data, "fold-in")
         cu, ci, cr = codes
-        alive = np.ones(len(cu), dtype=bool)
-
-        def listed(values):
-            return ", ".join(sorted(set(str(a) for a in values)))
-
-        bad_r = cr < 0
-        if bad_r.any():
-            logger.warning(f"The ratings {listed(labels[2][bad_r])} are in the fold-in set but weren't in the "
-                           f"train set so I'll remove them.")
-            alive &= ~bad_r
         both_new = alive & (cu < 0) & (ci < 0)
         if both_new.any():
-            logger.warning(f"The users {listed(labels[0][both_new])} are in the fold-in set with items "
-                           f"{listed(labels[1][both_new])} and neither was in the train set so I'll remove "
+            logger.warning(f"The users {_listed(labels[0][both_new])} are in the fold-in set with items "
+                           f"{_listed(labels[1][both_new])} and neither was in the train set so I'll remove "
                            f"those {int(both_new.sum())} rows.")
             alive &= ~both_new
         both_known = alive & (cu >= 0) & (ci >= 0)
         if both_known.any():
-            logger.warning(f"The users {listed(labels[0][both_known])} and items {listed(labels[1][both_known])} "
+            logger.warning(f"The users {_listed(labels[0][both_known])} and items {_listed(labels[1][both_known])} "
                            f"of {int(both_known.sum())} fold-in rows were in the train set so I'll ignore "
                            f"those rows: fit again to use them.")
             alive &= ~both_known
@@ -256,15 +270,36 @@ class DataHandler:
         for name, c, table, own, rows_name in (("users", 0, self.obs_dict, cu, "user_rows"),
                                               ("items", 1, self.items_dict, ci, "item_rows")):
             sel = alive & (own < 0)
-            new = sorted(set(labels[c][sel].tolist()))
-            rank = {s: k for k, s in enumerate(new)}
+            new, rank = self._rank_new(labels[c][sel])
             rows = np.stack([cu[sel], ci[sel], cr[sel]], axis=1).astype(np.int64).reshape(-1, 3)
-            rows[:, c] = [rank[s] for s in labels[c][sel].tolist()]
+            rows[:, c] = rank
             out[name], out[rows_name] = new, rows
         return out
 
+    def plan_refit(self, data):
+        """Host side of ``MMSBM.refit``: encode the rows of ``data`` (read by position, cells
+        ``str()``-ed) against the fitted dictionaries.  Nothing is changed; ``add_fold_in_ids``
+        records the new ids.
+
+        Known ids keep their codes; new users (items) get the codes after the existing ones, ranked
+        among themselves by ``sorted(set(str))``, as in ``plan_fold_in``.  Rows whose user and item
+        are both new are kept.  Rows with a rating value unseen in training are dropped with a
+        warning; if none is left this raises ``ValueError``.  Returns {"users", "items": new labels
+        in code order, "rows": int [N,3] (user, item, rating) in the order of ``data``}."""
+        codes, labels, alive = self._encode_known(data, "refit")
+        if not alive.any():
+            raise ValueError("refit data holds no row with a rating value the model knows")
+        out = {}
+        for name, c, table in (("users", 0, self.obs_dict), ("items", 1, self.items_dict)):
+            sel = alive & (codes[c] < 0)
+            out[name], rank = self._rank_new(labels[c][sel])
+            codes[c][sel] = len(table) + rank
+        out["rows"] = np.stack([c[alive] for c in codes], axis=1).astype(np.int64)
+        return out
+
     def add_fold_in_ids(self, users, items):
-        """Give the labels of ``plan_fold_in`` their codes after the existing ones."""
+        """Give the new labels of ``plan_fold_in`` / ``plan_refit`` their codes after the existing
+        ones."""
         for table, new in ((self.obs_dict, users), (self.items_dict, items)):
             base = len(table)
             for k, s in enumerate(new):

@@ -104,15 +104,21 @@ class MMSBM:
                 f"mmsbm_b200: with more than 32 groups on a side, ratings x groups must stay <= 1024 "
                 f"(got {n_levels} x {ld}); see INTEGRATION.md, 'Supported shapes'")
 
-    def _prepare_objects(self, train, build_engine=True):
+    def _prepare_objects(self, train, build_engine=True, counts=None):
         """Sizes, degree factors and the on-device index structure
         (replaces src/mmsbm.py:93-146; the O((U+I)N) scans become one GPU sort).
         ``build_engine=False`` (rating-sharded fits): no single-GPU index of all ratings is
-        built; the degrees come from a host bincount."""
-        self.ratings = list(np.unique(train[:, 2]))          # = sorted(set(train[:, 2])), src/mmsbm.py:95
+        built; the degrees come from a host bincount.  ``counts`` = (users, items, levels) when
+        the rows need not reach the top codes or every level (refit); by default they are
+        derived from the rows."""
+        if counts is None:
+            self.ratings = list(np.unique(train[:, 2]))      # = sorted(set(train[:, 2])), src/mmsbm.py:95
+            self.p = int(train[:, 0].max())
+            self.m = int(train[:, 1].max())
+        else:
+            self.ratings = list(range(counts[2]))
+            self.p, self.m = counts[0] - 1, counts[1] - 1
         self.r = max(self.ratings)
-        self.p = int(train[:, 0].max())
-        self.m = int(train[:, 1].max())
         self.train = train
         self._dims = {
             'n_samples': len(train),
@@ -207,24 +213,27 @@ class MMSBM:
             inits = [self._initial_parameters(s) for s in seeds]
         return tuple(np.stack([a[j] for a in inits]) for j in range(3))
 
-    def _run_batch(self, engine, seeds, run_ids):
+    def _run_batch(self, engine, seeds, run_ids, init=None, iterations=None):
+        """EM runs ``run_ids`` on ``engine``: from the seeded draws of ``seeds``, or from ``init`` =
+        stacked (theta0, eta0, pr0) when given; ``iterations`` defaults to ``self.iterations``."""
         import time
+        iterations = self.iterations if iterations is None else iterations
         t = time.perf_counter()
-        theta0, eta0, pr0 = self._initial_batch(seeds)
+        theta0, eta0, pr0 = self._initial_batch(seeds) if init is None else init
         t = self._tick("init_draws", t)
         engine.set_params(theta0, eta0, pr0)
         t = self._tick("params_h2d", t)
         if self.debug:
             done = 0
-            while done < self.iterations:
-                step = 1 if done == 0 else min(50, self.iterations - done)
+            while done < iterations:
+                step = 1 if done == 0 else min(50, iterations - done)
                 engine.run(step)
                 done += step
                 if (done - 1) % 50 == 0:
                     for i, lik in zip(run_ids, engine.likelihood()):
                         self.logger.debug(f"\nLikelihood at run {i} is {lik:.0f}")
         else:
-            engine.run(self.iterations)
+            engine.run(iterations)
         t = self._tick("em_iterations", t)
         lik = engine.likelihood()
         t = self._tick("likelihood", t)
@@ -375,6 +384,84 @@ class MMSBM:
         self.p, self.m = self.p + nu, self.m + ni
         self._index_cache = None
         return added
+
+    # ------------------------------------------------------------------------ refit
+    def refit(self, data, iterations=None, seed=0):
+        """Fit on ``data`` again, starting from this model's parameters instead of random draws.
+
+        ``data`` is the whole rating set the model should describe from now on -- normally the old
+        ratings plus the new ones, NOT only the new rows.  It is read by position like ``fit`` and
+        encoded against the model's dictionaries (DataHandler.plan_refit): known ids keep their
+        codes, new users and items get the codes after the existing ones (ranked among themselves by
+        ``sorted(set(str))``), rows with a rating value the model does not have are dropped with a
+        warning.  Run s starts from its current theta / eta / pr; new ids draw from
+        ``default_rng(SeedSequence(seed).spawn(S)[s])``: ``random((new users, K))`` then
+        ``random((new items, L))``, each row divided by max(its rows in ``data``, 1).  ``self.rng``
+        is not used.  ``iterations`` (default: ``self.iterations``) EM steps then run over all rows,
+        for every run.  Known ids without a row in ``data`` keep their parameters (with a warning);
+        a rating level without a row gets a zero pr slab, as in EM.  Calling ``fold_in(data)`` first
+        gives the new ids a fold-in start instead of a random one.
+
+        Afterwards ``results``, ``train`` and the degree factors describe ``data``, and
+        ``likelihood`` / ``predict`` / ``score`` / ``save`` / ``refit`` work as after ``fit``.
+        Returns {"users": [...], "items": [...]}: the labels added, in code order."""
+        import time
+        self._check_is_fitted()
+        iterations = self.iterations if iterations is None else int(iterations)
+        self.timings = {}
+        t = time.perf_counter()
+        plan = self.data_handler.plan_refit(data)
+        t = self._tick("encode_plan", t)
+        rows = plan["rows"]
+        S, K, L, R = len(self.results), self.user_groups, self.item_groups, self._dims['n_ratings']
+        U0, I0 = self.p + 1, self.m + 1
+        U, I = U0 + len(plan["users"]), I0 + len(plan["items"])
+        deg_u, deg_i = np.bincount(rows[:, 0], minlength=U), np.bincount(rows[:, 1], minlength=I)
+        du, di = np.maximum(deg_u[U0:], 1)[:, None], np.maximum(deg_i[I0:], 1)[:, None]
+        theta0, eta0 = np.empty((S, U, K)), np.empty((S, I, L))
+        for s, (res, child) in enumerate(zip(self.results, np.random.SeedSequence(seed).spawn(S))):
+            rng = np.random.default_rng(child)
+            theta0[s, :U0], theta0[s, U0:] = res["theta"], rng.random((U - U0, K)) / du
+            eta0[s, :I0], eta0[s, I0:] = res["eta"], rng.random((I - I0, L)) / di
+        pr0 = np.stack([res["pr"] for res in self.results])
+        absent_u, absent_i = np.flatnonzero(deg_u[:U0] == 0), np.flatnonzero(deg_i[:I0] == 0)
+        if len(absent_u) or len(absent_i):
+            self.logger.warning(f"{len(absent_u)} users and {len(absent_i)} items of the model have no rows in "
+                                f"the refit set so they keep their parameters.")
+        t = self._tick("init_draws", t)
+
+        rank, world = dist_info()
+        if world > 1 and self.shard == "ratings":
+            self._prepare_objects(rows, build_engine=False, counts=(U, I, R))
+            eng = ShardedEngine(rows, U, I, R, K, L)
+            every = list(range(S))
+            try:
+                done = self._run_batch(eng, None, every, init=(theta0, eta0, pr0), iterations=iterations)
+            finally:
+                eng.close()
+            results = [done[s] for s in every]
+        else:
+            self._prepare_objects(rows, counts=(U, I, R))
+            self._tick("rows_h2d_index_build", t)
+            mine = shard_runs(S, rank, world)
+            local = self._run_batch(self._engine, None, mine, init=(theta0[mine], eta0[mine], pr0[mine]),
+                                    iterations=iterations) if mine else {}
+            # EM leaves a zero row where an id has no rating: put the old rows back, on the device too
+            # when the engine still holds these runs for predict
+            if self._resident is not None:
+                import torch
+                e = self._engine
+                for absent, cur, init, width in ((absent_u, e.theta, theta0, K), (absent_i, e.eta, eta0, L)):
+                    if len(absent):
+                        cur[:, torch.from_numpy(absent).to(e.device), :width] = \
+                            torch.from_numpy(init[np.ix_(mine, absent)]).to(e.device)
+            results = gather_runs(local, S)
+        for s, res in enumerate(results):
+            res["theta"][absent_u] = theta0[s, absent_u]
+            res["eta"][absent_i] = eta0[s, absent_i]
+        self.results = results
+        self.data_handler.add_fold_in_ids(plan["users"], plan["items"])
+        return {"users": plan["users"], "items": plan["items"]}
 
     # ----------------------------------------------------------------------- cv_fit
     def _make_folds(self, data, folds):
