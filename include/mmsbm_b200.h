@@ -153,6 +153,31 @@ int mmsbm_em_run(const int32_t* useg_dev, const int32_t* uadj_dev, const int32_t
                  double* theta_a_dev, double* eta_a_dev, double* pr_a_dev,
                  double* theta_b_dev, double* eta_b_dev, double* pr_b_dev,
                  void* workspace_dev, size_t workspace_bytes, void* stream);
+/* EM until every run converges or ``max_iterations`` steps: the observed-data log-likelihood l
+ * (mmsbm_loglik) is taken at the start (l_0) and after min(j * check_every, max_iterations) steps
+ * (l_j, j = 1..checks, checks = ceil(max_iterations / check_every)).  Run s stops at the first
+ * check j >= 1 with |l_j - l_{j-1}| <= tol * |l_j|: its parameters are those after that check's
+ * step count, iterations_dev[s] is that count and converged_dev[s] is 1.  A run that never meets
+ * the rule ends after max_iterations steps with converged_dev[s] = 0.  loglik_dev [S][checks + 1]
+ * holds l_0..l_j of each run and NaN after its stop.  check_every must be even and >= 2, tol finite
+ * and >= 0.  A stopped run's results do not depend on the other runs of the batch.  On return the
+ * parameters of every run are in the _a buffers (_b is scratch).  Workspace:
+ * mmsbm_em_converge_workspace_bytes (the EM workspace, or the l workspace if larger, plus
+ * S * (U*ldk + I*ldl + K*L*R) doubles of snapshots).  SYNCHRONOUS, unlike the rest of this ABI:
+ * the call reads the schedule headers once and, per check, the count of runs still active (the next
+ * chunk of steps is already enqueued when it waits), and returns after synchronising ``stream``. */
+int mmsbm_em_converge_workspace_bytes(int64_t n_ratings, int32_t n_users, int32_t n_items, int32_t n_levels,
+                                      int32_t K, int32_t L, int32_t n_runs, size_t* bytes);
+int mmsbm_em_run_converge(const int32_t* useg_dev, const int32_t* uadj_dev, const int32_t* udeg_dev,
+                          const int32_t* iseg_dev, const int32_t* iadj_dev, const int32_t* ideg_dev,
+                          const int32_t* usched_dev, const int32_t* isched_dev,
+                          int64_t n_ratings, int32_t n_users, int32_t n_items, int32_t n_levels,
+                          int32_t K, int32_t L, int32_t n_runs,
+                          int32_t max_iterations, int32_t check_every, double tol,
+                          double* theta_a_dev, double* eta_a_dev, double* pr_a_dev,
+                          double* theta_b_dev, double* eta_b_dev, double* pr_b_dev,
+                          double* loglik_dev, int32_t* iterations_dev, int32_t* converged_dev,
+                          void* workspace_dev, size_t workspace_bytes, void* stream);
 /* post-all-reduce epilogue of a rating-sharded run: eta = n_eta / max(deg,1),
  * pr normalised over the rating axis (zero sums divide by one). In place. */
 int mmsbm_em_finalize(double* eta_dev, const int32_t* ideg_dev, int32_t n_items, int32_t L,
@@ -239,6 +264,18 @@ int mmsbm_likelihood(const int32_t* useg_dev, const int32_t* uadj_dev, const int
                      int32_t K, int32_t L, int32_t n_runs,
                      const double* theta_dev, const double* eta_dev, const double* pr_dev,
                      double* out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
+
+/* ---- the observed-data log-likelihood, the objective EM increases (the reference has none):
+ *      out_dev[s] = sum_n log max(sum_kl theta[u_n,k] eta[i_n,l] pr[k,l,r_n], eps), eps =
+ *      np.finfo(float).eps, for every shape mmsbm_em_step serves; usched_dev is required.
+ *      All runs at once; asynchronous, allocates nothing. ---------------------------------- */
+int mmsbm_loglik_workspace_bytes(int64_t n_ratings, int32_t n_users, int32_t n_items, int32_t n_levels,
+                                 int32_t K, int32_t L, int32_t n_runs, size_t* bytes);
+int mmsbm_loglik(const int32_t* useg_dev, const int32_t* uadj_dev, const int32_t* usched_dev,
+                 int64_t n_ratings, int32_t n_users, int32_t n_items, int32_t n_levels,
+                 int32_t K, int32_t L, int32_t n_runs,
+                 const double* theta_dev, const double* eta_dev, const double* pr_dev,
+                 double* out_dev, void* workspace_dev, size_t workspace_bytes, void* stream);
 
 /* ---- a6: rat[s][m][r], replaces prod_dist (src/kernels_numpy.py:86-97) ------------------ */
 int mmsbm_prod_dist(const int32_t* user_dev, const int32_t* item_dev, int64_t n_rows,

@@ -59,10 +59,14 @@ _PROTOS = {
     "mmsbm_em_run": (C.c_int, [_vp] * 8 + [_i64] + [_i32] * 7 + [_vp] * 6 + [_vp, _sz, _vp]),
     "mmsbm_fold_in_workspace_bytes": (C.c_int, [_i64] + [_i32] * 7 + [C.POINTER(_sz)]),
     "mmsbm_fold_in": (C.c_int, [_vp] * 3 + [_i64] + [_i32] * 8 + [_vp] * 3 + [_vp, _sz, _vp]),
+    "mmsbm_em_converge_workspace_bytes": (C.c_int, [_i64] + [_i32] * 6 + [C.POINTER(_sz)]),
+    "mmsbm_em_run_converge": (C.c_int, [_vp] * 8 + [_i64] + [_i32] * 8 + [C.c_double] + [_vp] * 9 + [_vp, _sz, _vp]),
     "mmsbm_em_finalize": (C.c_int, [_vp, _vp, _i32, _i32, _vp, _i32, _i32, _i32, _vp]),
     "mmsbm_likelihood_workspace_bytes": (C.c_int, [_i64] + [_i32] * 6 + [C.POINTER(_sz)]),
     "mmsbm_likelihood_min_workspace_bytes": (C.c_int, [_i64] + [_i32] * 6 + [C.POINTER(_sz)]),
     "mmsbm_likelihood": (C.c_int, [_vp, _vp, _vp, _i64] + [_i32] * 6 + [_vp] * 4 + [_vp, _sz, _vp]),
+    "mmsbm_loglik_workspace_bytes": (C.c_int, [_i64] + [_i32] * 6 + [C.POINTER(_sz)]),
+    "mmsbm_loglik": (C.c_int, [_vp, _vp, _vp, _i64] + [_i32] * 6 + [_vp] * 4 + [_vp, _sz, _vp]),
     "mmsbm_prod_dist": (C.c_int, [_vp, _vp, _i64] + [_i32] * 6 + [_vp] * 4 + [_vp]),
     "mmsbm_stats_workspace_bytes": (C.c_int, [_i64, _i32, C.POINTER(_sz)]),
     "mmsbm_predict_stats": (C.c_int, [_vp, _vp, _i64, _i32, _i32, _vp, _vp, _vp, _vp, _sz, _vp]),

@@ -59,12 +59,19 @@ int launch_finalize_pr(double* pr, int kl_total, int R, cudaStream_t st);
 
 // em_small.cu: a whole fit of a small one-run problem in one cooperative launch.  Returns
 // MMSBM_ERANGE when the shape (or the device, or MMSBM_COOP=0) is not served: take the other path.
+// long_segments: whether a schedule holds a segment cut into pieces (0/1) when the caller has read
+// the schedule headers, -1 to have them read here (one stream synchronisation).
 bool em_small_applicable(int64_t N, int R, int K, int L, int S);
 size_t em_small_partial_elems(int R, int K);
 int launch_em_small(const int32_t* useg, const int32_t* uadj, const int32_t* udeg, const int32_t* iseg,
                     const int32_t* iadj, const int32_t* ideg, const int32_t* usched, const int32_t* isched, int64_t N,
                     int U, int I, int R, int K, int L, int S, int iterations, double* theta_a, double* eta_a,
                     double* pr_a, double* theta_b, double* eta_b, double* pr_b, double* partial, size_t partial_elems,
-                    cudaStream_t st);
+                    cudaStream_t st, int long_segments = -1);
+
+// reductions.cu: observed-data log-likelihood of S runs (mmsbm_loglik without the argument checks)
+int launch_loglik(const int32_t* useg, const int32_t* uadj, const int32_t* usched, int64_t N, int U, int I,
+                  int R, int K, int L, int S, const double* theta, const double* eta, const double* pr,
+                  double* out, void* ws, size_t ws_bytes, cudaStream_t st);
 
 }  // namespace mmsbm

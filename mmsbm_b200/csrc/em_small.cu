@@ -322,7 +322,7 @@ int launch_em_small(const int32_t* useg, const int32_t* uadj, const int32_t* ude
                     const int32_t* iadj, const int32_t* ideg, const int32_t* usched, const int32_t* isched, int64_t N,
                     int U, int I, int R, int K, int L, int S, int iterations, double* theta_a, double* eta_a,
                     double* pr_a, double* theta_b, double* eta_b, double* pr_b, double* partial, size_t partial_elems,
-                    cudaStream_t st) {
+                    cudaStream_t st, int long_segments) {
   const int ldk = row_stride(K);
   if (!em_small_applicable(N, R, K, L, S) || iterations <= 0 || !partial) return MMSBM_ERANGE;
   if (env_int("MMSBM_COOP", 1) == 0) return MMSBM_ERANGE;
@@ -332,7 +332,8 @@ int launch_em_small(const int32_t* useg, const int32_t* uadj, const int32_t* ude
     return MMSBM_ERANGE;
   cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(st, &cap) != cudaSuccess || cap != cudaStreamCaptureStatusNone) return MMSBM_ERANGE;
-  {
+  if (long_segments > 0) return MMSBM_ERANGE;
+  if (long_segments < 0) {
     // a segment of more than MMSBM_PIECE_LEN ratings (heavy-tailed ids) would be walked by one CTA while the
     // rest of the grid waits at the barrier: such problems stay on the multi-kernel path, whose piece
     // schedule spreads the segment over the GPU.  The schedule headers say whether one exists (16 bytes

@@ -1172,6 +1172,286 @@ extern "C" int mmsbm_em_run(const int32_t* useg, const int32_t* uadj, const int3
   return 0;
 }
 
+// ---- EM to convergence ----------------------------------------------------------------------
+// Check j (j = 0 at the start, then after min(j*every, max_iterations) steps) evaluates l_j of
+// every run (launch_loglik); converge_latch_kernel applies the rule to the runs still active and
+// converge_copy_kernel snapshots the parameters of those that stop.  Latched runs keep being
+// computed by the batched kernels; nothing of theirs is written again, so their results do not
+// depend on the other runs.  The check index lives on the device, so one captured chunk (steps,
+// l, latch, snapshot) replays unchanged.
+namespace mmsbm {
+
+struct ConvState {
+  double* lik;        // [S] l of the current check
+  double* prev;       // [S] l of the run's previous check
+  int32_t* active;    // [S]
+  int32_t* stop;      // [S] 1: the run stops at the current check
+  int32_t* ctr;       // [0] index of the next check, [1] runs still active after it
+};
+
+__global__ void converge_init_kernel(ConvState c, double* trace, int32_t* iters, int32_t* conv, int S,
+                                     int ntr, int max_it) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < S * ntr) trace[t] = __longlong_as_double(0x7ff8000000000000ll);   // NaN: no entry
+  if (t < S) { c.active[t] = 1; iters[t] = max_it; conv[t] = 0; }
+  if (t == 0) { c.ctr[0] = 0; c.ctr[1] = S; }
+}
+
+__global__ void __launch_bounds__(256) converge_latch_kernel(ConvState c, double* trace, int32_t* iters,
+                                                             int32_t* conv, int S, int ntr, int every,
+                                                             int max_it, double tol) {
+  __shared__ int n_active;
+  const int j = c.ctr[0];
+  if (threadIdx.x == 0) n_active = 0;
+  __syncthreads();
+  int mine = 0;
+  for (int s = threadIdx.x; s < S; s += blockDim.x) {
+    int stop = 0;
+    if (c.active[s]) {
+      const double l = c.lik[s];
+      trace[(size_t)s * ntr + j] = l;
+      if (j > 0 && fabs(l - c.prev[s]) <= tol * fabs(l)) {
+        stop = 1;
+        c.active[s] = 0;
+        iters[s] = min(j * every, max_it);
+        conv[s] = 1;
+      } else {
+        c.prev[s] = l;
+        ++mine;
+      }
+    }
+    c.stop[s] = stop;
+  }
+  atomicAdd(&n_active, mine);   // an integer count: the order of the additions does not matter
+  __syncthreads();
+  if (threadIdx.x == 0) { c.ctr[0] = j + 1; c.ctr[1] = n_active; }
+}
+
+// dst <- src for the runs with pick[run] != 0: theta [U][ldk], eta [I][ldl] and pr [K*L*R] of a run
+struct RunCopy {
+  const double* src[3];
+  double* dst[3];
+  size_t n[3];        // doubles per run
+};
+__global__ void converge_copy_kernel(const RunCopy a, const int32_t* pick) {
+  const int run = blockIdx.y;
+  if (!pick[run]) return;
+  for (int t = 0; t < 3; ++t) {
+    const double* src = a.src[t] + (size_t)run * a.n[t];
+    double* dst = a.dst[t] + (size_t)run * a.n[t];
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < a.n[t]; i += (size_t)gridDim.x * blockDim.x)
+      dst[i] = src[i];
+  }
+}
+
+static int launch_run_copy(const RunCopy& a, const int32_t* pick, int S, cudaStream_t st) {
+  const size_t most = a.n[0] > a.n[1] ? (a.n[0] > a.n[2] ? a.n[0] : a.n[2]) : (a.n[1] > a.n[2] ? a.n[1] : a.n[2]);
+  const size_t want = (most + 255) / 256, cap = (size_t)sm_count() * 4;
+  converge_copy_kernel<<<dim3((unsigned)(want < cap ? want : cap), S), 256, 0, st>>>(a, pick);
+  MMSBM_LAUNCH_CHECK("converge_copy_kernel");
+  return 0;
+}
+
+// the EM workspace and the l workspace share one region (they are never in use at the same time)
+static size_t converge_shared_bytes(int64_t N, int U, int I, int R, int K, int L, int S) {
+  size_t em = 0, lk = 0;
+  mmsbm_em_workspace_bytes(N, U, I, R, K, L, S, &em);
+  mmsbm_loglik_workspace_bytes(N, U, I, R, K, L, S, &lk);
+  return em > lk ? em : lk;
+}
+
+}  // namespace mmsbm
+
+extern "C" int mmsbm_em_converge_workspace_bytes(int64_t N, int32_t U, int32_t I, int32_t R, int32_t K,
+                                                 int32_t L, int32_t S, size_t* bytes) {
+  MMSBM_REQUIRE(bytes && N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
+                "mmsbm_em_converge_workspace_bytes: bad argument");
+  const size_t snap = (size_t)S * ((size_t)U * row_stride(K) + (size_t)I * row_stride(L) + (size_t)K * L * R);
+  *bytes = converge_shared_bytes(N, U, I, R, K, L, S) + align_up(snap * 8) + 2 * align_up((size_t)S * 8) +
+           2 * align_up((size_t)S * 4) + align_up(2 * 4) + 256;
+  return 0;
+}
+
+extern "C" int mmsbm_em_run_converge(const int32_t* useg, const int32_t* uadj, const int32_t* udeg,
+                                     const int32_t* iseg, const int32_t* iadj, const int32_t* ideg,
+                                     const int32_t* usched, const int32_t* isched,
+                                     int64_t N, int32_t U, int32_t I, int32_t R, int32_t K, int32_t L, int32_t S,
+                                     int32_t max_iterations, int32_t check_every, double tol,
+                                     double* theta_a, double* eta_a, double* pr_a,
+                                     double* theta_b, double* eta_b, double* pr_b,
+                                     double* loglik, int32_t* iterations, int32_t* converged,
+                                     void* ws, size_t ws_bytes, void* stream) {
+  MMSBM_REQUIRE(useg && uadj && udeg && iseg && iadj && ideg && usched && isched && theta_a && eta_a && pr_a &&
+                    theta_b && eta_b && pr_b && loglik && iterations && converged && ws, MMSBM_EINVAL,
+                "mmsbm_em_run_converge: null pointer");
+  MMSBM_REQUIRE(N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
+                "mmsbm_em_run_converge: bad size");
+  MMSBM_REQUIRE(K <= 256 && L <= 256 && R <= 31, MMSBM_ERANGE,
+                "mmsbm_em_run_converge: K, L <= 256 and R <= 31 supported (K=%d L=%d R=%d)", K, L, R);
+  MMSBM_REQUIRE(max_iterations >= 0 && check_every >= 2 && check_every % 2 == 0, MMSBM_EINVAL,
+                "mmsbm_em_run_converge: max_iterations >= 0 and an even check_every >= 2 required (%d, %d)",
+                max_iterations, check_every);
+  MMSBM_REQUIRE(tol >= 0.0 && tol <= 1.7976931348623157e308, MMSBM_EINVAL,
+                "mmsbm_em_run_converge: tol must be finite and >= 0");
+  size_t need = 0;
+  mmsbm_em_converge_workspace_bytes(N, U, I, R, K, L, S, &need);
+  MMSBM_REQUIRE(ws_bytes >= need, MMSBM_ENOMEM, "mmsbm_em_run_converge: workspace too small (%zu < %zu)",
+                ws_bytes, need);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  const int ldk = row_stride(K), ldl = row_stride(L);
+  const int c = check_every, full = max_iterations / c, rem = max_iterations - full * c;
+  const int checks = full + (rem > 0 ? 1 : 0), ntr = checks + 1;
+  const size_t shared = converge_shared_bytes(N, U, I, R, K, L, S);
+  const size_t n_th = (size_t)U * ldk, n_et = (size_t)I * ldl, n_pr = (size_t)K * L * R;
+  Arena arena(static_cast<char*>(ws) + shared, ws_bytes - shared);
+  double* snap = arena.take<double>((size_t)S * (n_th + n_et + n_pr));
+  ConvState cs;
+  cs.lik = arena.take<double>(S);
+  cs.prev = arena.take<double>(S);
+  cs.active = arena.take<int32_t>(S);
+  cs.stop = arena.take<int32_t>(S);
+  cs.ctr = arena.take<int32_t>(2);
+  MMSBM_REQUIRE(snap && cs.lik && cs.prev && cs.active && cs.stop && cs.ctr, MMSBM_ENOMEM,
+                "mmsbm_em_run_converge: workspace too small");
+  double* snap3[3] = {snap, snap + (size_t)S * n_th, snap + (size_t)S * (n_th + n_et)};
+
+  // launch strategy, decided once per call as in mmsbm_em_run: the schedule headers (16 bytes each)
+  int32_t hu[4] = {0, 0, 1, 0}, hi[4] = {0, 0, 1, 0};
+  MMSBM_CUDA(cudaMemcpyAsync(hu, usched, sizeof(hu), cudaMemcpyDeviceToHost, st));
+  MMSBM_CUDA(cudaMemcpyAsync(hi, isched, sizeof(hi), cudaMemcpyDeviceToHost, st));
+  MMSBM_CUDA(cudaStreamSynchronize(st));
+  const bool has_long = hu[2] != 0 || hi[2] != 0;
+  const size_t part_elems = em_small_partial_elems(R, K);
+  const size_t main_bytes = em_main_bytes(em_dims(N, U, I, R, K, L, S));
+  bool coop = checks > 0 && em_small_applicable(N, R, K, L, S) && !has_long && shared >= main_bytes + part_elems * 8;
+  Overlap ov;
+  const bool small = (double)N * S < 5.0e7;
+  const bool overlap = checks > 0 && getenv("MMSBM_NO_OVERLAP") == nullptr;
+  ov.no_long_u = hu[2] == 0;
+  ov.no_long_i = hi[2] == 0;
+  struct Resources {
+    cudaStream_t st;
+    Overlap& o;
+    cudaEvent_t done[2] = {nullptr, nullptr};
+    int32_t* host = nullptr;                    // pinned: the count of active runs, one slot per check in flight
+    cudaGraphExec_t exec = nullptr;
+    ~Resources() {
+      cudaStreamSynchronize(st);                // nothing may still write to `host`
+      if (exec) cudaGraphExecDestroy(exec);
+      for (auto& e : done) if (e) cudaEventDestroy(e);
+      if (host) cudaFreeHost(host);
+      for (auto& e : o.e) if (e) cudaEventDestroy(e);
+      if (o.side) cudaStreamDestroy(o.side);
+    }
+  } res{st, ov};
+  if (overlap) {
+    MMSBM_CUDA(cudaStreamCreateWithFlags(&ov.side, cudaStreamNonBlocking));
+    for (auto& e : ov.e) MMSBM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    ov.two_branch = small && getenv("MMSBM_FORCE_OVERLAP") == nullptr;
+  }
+  for (auto& e : res.done) MMSBM_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+  MMSBM_CUDA(cudaHostAlloc(reinterpret_cast<void**>(&res.host), 2 * sizeof(int32_t), cudaHostAllocDefault));
+
+  double* a3[3] = {theta_a, eta_a, pr_a};
+  double* b3[3] = {theta_b, eta_b, pr_b};
+  // l of the parameters in p3, then the latch and the snapshots of the runs that stop
+  auto check = [&](double* const* p3) {
+    int rc = launch_loglik(useg, uadj, usched, N, U, I, R, K, L, S, p3[0], p3[1], p3[2], cs.lik, ws, shared, st);
+    if (rc) return rc;
+    converge_latch_kernel<<<1, 256, 0, st>>>(cs, loglik, iterations, converged, S, ntr, c, max_iterations, tol);
+    MMSBM_LAUNCH_CHECK("converge_latch_kernel");
+    const RunCopy cp{{p3[0], p3[1], p3[2]}, {snap3[0], snap3[1], snap3[2]}, {n_th, n_et, n_pr}};
+    return launch_run_copy(cp, cs.stop, S, st);
+  };
+  // `steps` EM steps from the _a buffers (they end in _b when `steps` is odd), then a check
+  auto chunk = [&](int steps) {
+    int rc = MMSBM_ERANGE;
+    if (coop) {
+      rc = launch_em_small(useg, uadj, udeg, iseg, iadj, ideg, usched, isched, N, U, I, R, K, L, S, steps,
+                           theta_a, eta_a, pr_a, theta_b, eta_b, pr_b,
+                           reinterpret_cast<double*>(static_cast<char*>(ws) + main_bytes), part_elems, st, 0);
+      if (rc == MMSBM_ERANGE) coop = false;     // device or stream not served: the multi-kernel path
+      else if (rc) return rc;
+    }
+    if (!coop) {
+      for (int it = 0; it < steps; ++it) {
+        const bool fwd = (it & 1) == 0;
+        rc = em_step_impl(useg, uadj, udeg, iseg, iadj, ideg, usched, isched, N, U, I, R, K, L, S,
+                          fwd ? theta_a : theta_b, fwd ? eta_a : eta_b, fwd ? pr_a : pr_b,
+                          fwd ? theta_b : theta_a, fwd ? eta_b : eta_a, fwd ? pr_b : pr_a, 0, ws, shared,
+                          stream, nullptr, overlap ? &ov : nullptr);
+        if (rc) return rc;
+      }
+    }
+    return check((steps & 1) ? b3 : a3);
+  };
+
+  {
+    const int t = S * ntr;
+    converge_init_kernel<<<(t + 255) / 256, 256, 0, st>>>(cs, loglik, iterations, converged, S, ntr, max_iterations);
+    MMSBM_LAUNCH_CHECK("converge_init_kernel");
+    if (int rc = check(a3)) return rc;          // l_0
+  }
+  int per_chunk = 0;
+  auto enqueue = [&](int j) {                  // check j >= 1, then the count of runs still active
+    int rc;
+    if (res.exec && j <= full) {
+      MMSBM_CUDA(cudaGraphLaunch(res.exec, st));
+      count_launch(per_chunk);
+    } else if ((rc = chunk(j <= full ? c : rem))) {
+      return rc;
+    }
+    MMSBM_CUDA(cudaMemcpyAsync(res.host + (j & 1), cs.ctr + 1, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    MMSBM_CUDA(cudaEventRecord(res.done[j & 1], st));
+    return 0;
+  };
+  int enqueued = 0;
+  if (checks > 0) {
+    if (int rc = enqueue(1)) return rc;
+    enqueued = 1;
+    // launch-bound sizes: capture one chunk into a CUDA graph (the first ran uncaptured and set the
+    // function attributes) and replay it for the other full chunks
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    if (!coop && small && full >= 3 && st != nullptr && getenv("MMSBM_NO_GRAPH") == nullptr &&
+        cudaStreamIsCapturing(st, &cap) == cudaSuccess && cap == cudaStreamCaptureStatusNone) {
+      cudaGraph_t graph = nullptr;
+      const int64_t l0 = mmsbm_launch_count();
+      MMSBM_CUDA(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+      int rc = chunk(c);
+      cudaError_t e = cudaStreamEndCapture(st, &graph);
+      per_chunk = (int)(mmsbm_launch_count() - l0);
+      count_launch(-per_chunk);                // the capture itself launched nothing
+      if (rc == 0 && e == cudaSuccess && graph) e = cudaGraphInstantiate(&res.exec, graph, 0);
+      if (graph) cudaGraphDestroy(graph);
+      if (rc) return rc;
+      if (e != cudaSuccess) {
+        res.exec = nullptr;
+        (void)cudaGetLastError();              // graph path unavailable: plain launches
+      }
+    }
+  }
+  // one chunk of lookahead: chunk j+1 is enqueued before the host waits for the count of check j
+  for (int j = 1; j <= checks; ++j) {
+    if (j < checks) {
+      if (int rc = enqueue(j + 1)) return rc;
+      enqueued = j + 1;
+    }
+    MMSBM_CUDA(cudaEventSynchronize(res.done[j & 1]));
+    if (res.host[j & 1] == 0) break;
+  }
+  // every run's parameters into _a: the last chunk may have ended in _b, latched runs from their snapshots
+  const int steps_done = enqueued <= full ? enqueued * c : max_iterations;
+  if (steps_done & 1)
+    for (int t = 0; t < 3; ++t) {
+      const size_t n = (size_t)S * (t == 0 ? n_th : t == 1 ? n_et : n_pr);
+      MMSBM_CUDA(cudaMemcpyAsync(a3[t], b3[t], n * 8, cudaMemcpyDeviceToDevice, st));
+    }
+  const RunCopy back{{snap3[0], snap3[1], snap3[2]}, {theta_a, eta_a, pr_a}, {n_th, n_et, n_pr}};
+  if (int rc = launch_run_copy(back, converged, S, st)) return rc;
+  MMSBM_CUDA(cudaStreamSynchronize(st));
+  return 0;
+}
+
 extern "C" int mmsbm_em_finalize(double* eta, const int32_t* ideg, int32_t I, int32_t L, double* pr,
                                  int32_t K, int32_t R, int32_t S, void* stream) {
   MMSBM_REQUIRE(eta && ideg && pr && I > 0 && L > 0 && K > 0 && R > 0 && S > 0, MMSBM_EINVAL,

@@ -196,29 +196,35 @@ __global__ void __launch_bounds__(256) lik_user_tables_kernel(const double* __re
 
 struct LikPassArgs {
   const int32_t* useg; const int32_t* uadj; const int32_t* sched;
-  const double* e2;       // [runs][I][2][NBp]
-  const double* W;        // [runs][U][R*NBp]
-  const double* A;
+  const double* e2;       // [runs][I][2][NBp]; OBS: eta [runs][I][ld]
+  const double* W;        // [runs][U][R*NBp]; OBS: [runs][U][R*ld]
+  const double* A;        // (not read by OBS)
   double* partial;        // [runs][pmax]
   int64_t pmax;
   int U, I, R;
+  int ld;                 // OBS: row stride of eta (NBp when G < 8, any multiple of 4 >= 32 when G == 8)
 };
 
 // One warp per piece; groups of G lanes own a rating (lane q holds doubles 4q..4q+3 of both rows).
-template <int G>
-__global__ void __launch_bounds__(256) lik_pass_kernel(const LikPassArgs P) {
+// OBS: the observed-data log-likelihood sum_n log max(S_n, eps) instead: only W and eta rows are
+// read (half the bytes per rating), and rows wider than 32 doubles are walked in slices of 32
+// (lane q of the 8-lane group holds doubles 32c+4q..32c+4q+3 of slice c).
+// One body, two kernels (lik_pass_kernel, loglik_pass_kernel), so each form keeps its own name.
+template <int G, bool OBS>
+__device__ __forceinline__ void lik_pass_body(const LikPassArgs& P) {
   constexpr int RPS = 32 / G, UN = (G == 1) ? 1 : 2, SLOTS = UN * RPS, NBp = 4 * G;
   static_assert(SLOTS <= 32, "a chunk's ids must fit one 32-lane load");
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int grp = lane / G, q = lane - grp * G;
   const bool lane_on = grp < RPS;
   const int qoff = lane_on ? 4 * q : 0;
-  const int run = blockIdx.y, R = P.R, RNB = R * NBp;
+  const int LD = OBS ? P.ld : NBp, nsl = (LD + NBp - 1) / NBp;
+  const int run = blockIdx.y, R = P.R, RNB = R * LD;
   const GroupSum<G> group_sum(grp * G, q);
   const int32_t* piece_seg = P.sched + 4;
   const int32_t* piece_idx = piece_seg + P.pmax;
   const int n_pieces = __ldg(P.sched);
-  const double* e2 = P.e2 + (size_t)run * P.I * 2 * NBp;
+  const double* e2 = P.e2 + (size_t)run * P.I * (OBS ? 1 : 2) * LD;
   for (int p = blockIdx.x * (blockDim.x >> 5) + warp; p < n_pieces; p += gridDim.x * (blockDim.x >> 5)) {
     const int sg = __ldg(piece_seg + p), pidx = __ldg(piece_idx + p);
     MMSBM_DEV_CHECK(sg >= 0 && sg < P.U);
@@ -233,11 +239,45 @@ __global__ void __launch_bounds__(256) lik_pass_kernel(const LikPassArgs P) {
     for (int r = 0; r < R; ++r) {
       const int le = min(end, __shfl_sync(kFull, bend, r + 1));
       if (lo >= le) continue;
-      const double4_t wr = ldg256(wrow + r * NBp + qoff), ar = ldg256(arow + r * NBp + qoff);
+      const double* wr_row = wrow + r * LD;
+      const double4_t wr = ldg256(wr_row + qoff);
+      double4_t ar{0.0, 0.0, 0.0, 0.0};
+      if constexpr (!OBS) ar = ldg256(arow + r * NBp + qoff);
       for (int base = lo; base < le; base += SLOTS) {
         const int cnt = min(SLOTS, le - base);
         int ids = 0;
         if (lane < cnt) ids = __ldg(P.uadj + base + lane);
+        if constexpr (OBS) {
+          int id[UN];
+          double4_t e[UN];
+          double sv[UN];
+#pragma unroll
+          for (int un = 0; un < UN; ++un) {
+            const int sl = un * RPS + grp;
+            id[un] = __shfl_sync(kFull, ids, sl & 31);
+            if (sl >= cnt) id[un] = 0;
+            MMSBM_DEV_CHECK(id[un] >= 0 && id[un] < P.I);
+            e[un] = ldg256(e2 + (size_t)id[un] * LD + qoff);
+          }
+#pragma unroll
+          for (int un = 0; un < UN; ++un) {
+            double s = fma(e[un].x, wr.x, fma(e[un].y, wr.y, fma(e[un].z, wr.z, e[un].w * wr.w)));
+            if constexpr (G == 8) {                          // rows wider than 32 doubles
+              for (int c = 1; c < nsl; ++c) {
+                const int off = c * NBp + qoff;
+                if (off < LD) {
+                  const double4_t ec = ldg256(e2 + (size_t)id[un] * LD + off), wc = ldg256(wr_row + off);
+                  s = fma(ec.x, wc.x, fma(ec.y, wc.y, fma(ec.z, wc.z, fma(ec.w, wc.w, s))));
+                }
+              }
+            }
+            sv[un] = group_sum(s);
+          }
+#pragma unroll
+          for (int un = 0; un < UN; ++un)
+            if (lane_on && q == 0 && un * RPS + grp < cnt) acc += log(fmax(sv[un], kEps));
+          continue;
+        }
         double4_t e[UN], el[UN];
 #pragma unroll
         for (int un = 0; un < UN; ++un) {
@@ -265,6 +305,12 @@ __global__ void __launch_bounds__(256) lik_pass_kernel(const LikPassArgs P) {
     if (lane == 0) P.partial[(size_t)run * P.pmax + p] = acc;
   }
 }
+
+template <int G>
+__global__ void __launch_bounds__(256) lik_pass_kernel(const LikPassArgs P) { lik_pass_body<G, false>(P); }
+
+template <int G>
+__global__ void __launch_bounds__(256) loglik_pass_kernel(const LikPassArgs P) { lik_pass_body<G, true>(P); }
 
 __global__ void __launch_bounds__(256) sum_partials_kernel(const double* partial, int n, double* out) {
   __shared__ double sm[256];
@@ -529,7 +575,7 @@ static int likelihood_factorised(const int32_t* useg, const int32_t* uadj, const
       case 32: rc = launch_lik_tables<32>(theta, pr, W, A, U, K, L, R, run0, n, st); break;
     }
     if (rc) return rc;
-    LikPassArgs a{useg, uadj, usched, e2, W, A, partial + (size_t)run0 * pmax, pmax, U, I, R};
+    LikPassArgs a{useg, uadj, usched, e2, W, A, partial + (size_t)run0 * pmax, pmax, U, I, R, ldl};
     const int64_t want = (pmax + 7) / 8;
     const int64_t cap = (int64_t)sm_count() * 16;
     const dim3 grid((unsigned)(want < cap ? want : cap), n);
@@ -583,6 +629,82 @@ extern "C" int mmsbm_likelihood(const int32_t* useg, const int32_t* uadj, const 
   sum_partials_kernel<<<S, 256, 0, st>>>(partial, nw, out);
   MMSBM_LAUNCH_CHECK("sum_partials_kernel");
   return 0;
+}
+
+// ---- observed-data log-likelihood ----------------------------------------------------------
+// l = sum_n log max(S_n, eps), S_n = sum_kl theta_uk eta_il p_klr = <W_{u,r}, eta_i>: the EM
+// objective (it never decreases from one EM step to the next).  W = theta x Pw comes from the EM
+// step's own contraction (prep_p_kernel + launch_w, every admitted shape); the by-user pass of the
+// factorised likelihood then gathers one eta row per rating, with the same piece schedule and the
+// same fixed-order two-stage sum.  All runs at once.
+static size_t loglik_bytes(int64_t N, int U, int R, int K, int L, int S) {
+  const size_t ldk = row_stride(K), ldl = row_stride(L);
+  return 4 * align_up((size_t)S * ldk * ldl * R * 8) + align_up((size_t)S * U * R * ldl * 8) +
+         align_up((size_t)S * lik_pmax(N, U) * 8) + 256;
+}
+
+namespace mmsbm {
+int launch_loglik(const int32_t* useg, const int32_t* uadj, const int32_t* usched, int64_t N, int U, int I,
+                  int R, int K, int L, int S, const double* theta, const double* eta, const double* pr,
+                  double* out, void* ws, size_t ws_bytes, cudaStream_t st) {
+  const int ldk = row_stride(K), ldl = row_stride(L), rnb = R * ldl;
+  const int64_t pmax = lik_pmax(N, U);
+  MMSBM_REQUIRE(pmax <= 0x7fffffff, MMSBM_ERANGE, "mmsbm_loglik: too many pieces");
+  Arena arena(ws, ws_bytes);
+  const size_t p_elems = (size_t)S * ldk * ldl * R;
+  double* pw = arena.take<double>(p_elems);                  // user-side operand layout (the one used)
+  double* pn = arena.take<double>(p_elems);
+  double* pwi = arena.take<double>(p_elems);
+  double* pni = arena.take<double>(p_elems);
+  double* W = arena.take<double>((size_t)S * U * rnb);
+  double* partial = arena.take<double>((size_t)S * pmax);
+  MMSBM_REQUIRE(pw && pn && pwi && pni && W && partial, MMSBM_ENOMEM, "mmsbm_loglik: workspace too small (%zu)",
+                ws_bytes);
+  int rc;
+  if ((rc = launch_prep_p(pr, K, L, R, ldk, ldl, S, pw, pn, pwi, pni, st))) return rc;
+  if ((rc = launch_w(theta, pw, W, U, ldk, rnb, S, st))) return rc;
+  MMSBM_CUDA(cudaMemsetAsync(partial, 0, (size_t)S * pmax * 8, st));
+  LikPassArgs a{useg, uadj, usched, eta, W, nullptr, partial, pmax, U, I, R, ldl};
+  const int64_t want = (pmax + 7) / 8;
+  const int64_t cap = (int64_t)sm_count() * 16;
+  const dim3 grid((unsigned)(want < cap ? want : cap), S);
+  switch (ldl < 32 ? ldl / 4 : 8) {
+    case 1: loglik_pass_kernel<1><<<grid, 256, 0, st>>>(a); break;
+    case 2: loglik_pass_kernel<2><<<grid, 256, 0, st>>>(a); break;
+    case 3: loglik_pass_kernel<3><<<grid, 256, 0, st>>>(a); break;
+    case 4: loglik_pass_kernel<4><<<grid, 256, 0, st>>>(a); break;
+    case 5: loglik_pass_kernel<5><<<grid, 256, 0, st>>>(a); break;
+    case 6: loglik_pass_kernel<6><<<grid, 256, 0, st>>>(a); break;
+    case 7: loglik_pass_kernel<7><<<grid, 256, 0, st>>>(a); break;
+    default: loglik_pass_kernel<8><<<grid, 256, 0, st>>>(a); break;
+  }
+  MMSBM_LAUNCH_CHECK("loglik_pass_kernel");
+  sum_partials_kernel<<<S, 256, 0, st>>>(partial, (int)pmax, out);
+  MMSBM_LAUNCH_CHECK("sum_partials_kernel");
+  return 0;
+}
+}  // namespace mmsbm
+
+extern "C" int mmsbm_loglik_workspace_bytes(int64_t N, int32_t U, int32_t I, int32_t R, int32_t K, int32_t L,
+                                            int32_t S, size_t* bytes) {
+  MMSBM_REQUIRE(bytes && N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
+                "mmsbm_loglik_workspace_bytes: bad argument");
+  *bytes = loglik_bytes(N, U, R, K, L, S);
+  return 0;
+}
+
+extern "C" int mmsbm_loglik(const int32_t* useg, const int32_t* uadj, const int32_t* usched, int64_t N,
+                            int32_t U, int32_t I, int32_t R, int32_t K, int32_t L, int32_t S,
+                            const double* theta, const double* eta, const double* pr, double* out,
+                            void* ws, size_t ws_bytes, void* stream) {
+  MMSBM_REQUIRE(useg && uadj && usched && theta && eta && pr && out && ws, MMSBM_EINVAL,
+                "mmsbm_loglik: null pointer");
+  MMSBM_REQUIRE(U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0 && N >= 0, MMSBM_EINVAL,
+                "mmsbm_loglik: bad size");
+  MMSBM_REQUIRE(K <= 256 && L <= 256 && R <= 31, MMSBM_ERANGE,
+                "mmsbm_loglik: K, L <= 256 and R <= 31 supported (K=%d L=%d R=%d)", K, L, R);
+  return launch_loglik(useg, uadj, usched, N, U, I, R, K, L, S, theta, eta, pr, out, ws, ws_bytes,
+                       static_cast<cudaStream_t>(stream));
 }
 
 extern "C" int mmsbm_prod_dist(const int32_t* user, const int32_t* item, int64_t M, int32_t U,

@@ -293,6 +293,51 @@ class Engine:
     def likelihood(self):
         return self.likelihood_device().cpu().numpy()
 
+    def loglik_device(self):
+        """Observed-data log-likelihood of every run, sum_n log max(sum_kl theta eta pr, eps): the
+        objective EM increases.  [S] float64 on the device."""
+        self._need_ratings()
+        out = self._empty(self.S, torch.float64)
+        dims = (self.N, self.U, self.I, self.R, self.K, self.L, self.S)
+        need = _lib.C.c_size_t(0)
+        _lib.check(self.lib.mmsbm_loglik_workspace_bytes(*dims, _lib.C.byref(need)), "loglik_workspace_bytes")
+        ws = self._bytes(need.value)
+        _lib.check(self.lib.mmsbm_loglik(
+            self.useg.data_ptr(), self.uadj.data_ptr(), self.usched.data_ptr(), *dims,
+            self.theta.data_ptr(), self.eta.data_ptr(), self.pr.data_ptr(),
+            out.data_ptr(), ws.data_ptr(), need.value, self._stream()), "loglik")
+        ws.record_stream(torch.cuda.current_stream(self.device))
+        return out[:self.S]
+
+    def loglik(self):
+        return self.loglik_device().cpu().numpy()
+
+    def run_converge(self, max_iterations, tol, check_every=10):
+        """EM until each run's log-likelihood changes by at most ``tol`` (relative) between two
+        checks ``check_every`` steps apart, or ``max_iterations`` steps (mmsbm_em_run_converge).
+        The final parameters of every run are left in theta / eta / pr.  Returns numpy
+        (iterations [S] int, converged [S] bool, trace [S, checks + 1]): the log-likelihood at
+        each check, NaN after the run's stop.  Synchronous."""
+        self._need_ratings()
+        max_iterations, check_every = int(max_iterations), int(check_every)
+        checks = -(-max_iterations // check_every) if max_iterations > 0 else 0
+        dims = (self.N, self.U, self.I, self.R, self.K, self.L, self.S)
+        need = _lib.C.c_size_t(0)
+        _lib.check(self.lib.mmsbm_em_converge_workspace_bytes(*dims, _lib.C.byref(need)),
+                   "em_converge_workspace_bytes")
+        ws = self._bytes(need.value)
+        trace = torch.empty((self.S, checks + 1), dtype=torch.float64, device=self.device)
+        iters = self._empty(self.S, torch.int32)
+        conv = self._empty(self.S, torch.int32)
+        a, b = (self.theta, self.eta, self.pr), self._alt
+        _lib.check(self.lib.mmsbm_em_run_converge(
+            *self._graph_args(), *dims, max_iterations, check_every, float(tol),
+            a[0].data_ptr(), a[1].data_ptr(), a[2].data_ptr(), b[0].data_ptr(), b[1].data_ptr(), b[2].data_ptr(),
+            trace.data_ptr(), iters.data_ptr(), conv.data_ptr(), ws.data_ptr(), need.value, self._stream()),
+            "em_run_converge")
+        return (iters.cpu().numpy()[:self.S].astype(np.int64), conv.cpu().numpy()[:self.S] != 0,
+                trace.cpu().numpy())
+
     def prod_dist_device(self, test):
         """rat [S,M,R] on the device for int [M,3] (or [M,2]) test rows."""
         test = np.asarray(test)

@@ -39,7 +39,7 @@ class MMSBM:
     seed : int or None
         Seed of the parent generator; run s uses the s-th SeedSequence child.
     debug : bool
-        Log the likelihood every 50 iterations.
+        Log the likelihood every 50 iterations (with ``tol``: the log-likelihood of every check).
     backend : str, default="auto"
         "auto" or "b200".  There is no CPU backend.
     shard : str, default="runs"  (extension; only matters under torch.distributed)
@@ -213,9 +213,24 @@ class MMSBM:
             inits = [self._initial_parameters(s) for s in seeds]
         return tuple(np.stack([a[j] for a in inits]) for j in range(3))
 
-    def _run_batch(self, engine, seeds, run_ids, init=None, iterations=None):
+    def _check_convergence_args(self, tol, check_every):
+        """The stopping rule's arguments, checked before any GPU work."""
+        if tol is not None:
+            if isinstance(tol, bool) or not isinstance(tol, (int, float, np.integer, np.floating)) \
+                    or not np.isfinite(tol) or tol < 0:
+                raise ValueError(f"tol must be a finite number >= 0 or None (got {tol!r})")
+            if dist_info()[1] > 1 and self.shard == "ratings":
+                raise ValueError("tol is not supported with shard='ratings' under torch.distributed; "
+                                 "use shard='runs' or a fixed iteration count")
+        if isinstance(check_every, bool) or not isinstance(check_every, (int, np.integer)) \
+                or check_every < 2 or check_every % 2:
+            raise ValueError(f"check_every must be an even integer >= 2 (got {check_every!r})")
+
+    def _run_batch(self, engine, seeds, run_ids, init=None, iterations=None, tol=None, check_every=10):
         """EM runs ``run_ids`` on ``engine``: from the seeded draws of ``seeds``, or from ``init`` =
-        stacked (theta0, eta0, pr0) when given; ``iterations`` defaults to ``self.iterations``."""
+        stacked (theta0, eta0, pr0) when given; ``iterations`` defaults to ``self.iterations``.
+        With ``tol``, ``iterations`` is the maximum and each run stops on its own at convergence
+        (Engine.run_converge); its result then also holds "iterations", "converged" and "loglik"."""
         import time
         iterations = self.iterations if iterations is None else iterations
         t = time.perf_counter()
@@ -223,7 +238,18 @@ class MMSBM:
         t = self._tick("init_draws", t)
         engine.set_params(theta0, eta0, pr0)
         t = self._tick("params_h2d", t)
-        if self.debug:
+        conv = None
+        if tol is not None:
+            n_it, converged, trace = engine.run_converge(iterations, tol, check_every)
+            conv = {}
+            for j, i in enumerate(run_ids):
+                checks = trace[j][~np.isnan(trace[j])]
+                conv[i] = {"iterations": int(n_it[j]), "converged": bool(converged[j]), "loglik": checks}
+                if self.debug:
+                    for c, v in enumerate(checks):
+                        self.logger.debug(f"\nLog-likelihood at run {i} after "
+                                          f"{min(c * check_every, iterations)} iterations is {v:.6f}")
+        elif self.debug:
             done = 0
             while done < iterations:
                 step = 1 if done == 0 else min(50, iterations - done)
@@ -240,11 +266,24 @@ class MMSBM:
         theta, eta, pr = engine.get_params()
         t = self._tick("results_d2h", t)
         self._resident = list(run_ids) if engine is self._engine else None
-        return {i: {"likelihood": np.float64(lik[j]), "pr": pr[j], "theta": theta[j], "eta": eta[j]}
-                for j, i in enumerate(run_ids)}
+        out = {i: {"likelihood": np.float64(lik[j]), "pr": pr[j], "theta": theta[j], "eta": eta[j]}
+               for j, i in enumerate(run_ids)}
+        if conv is not None:
+            for i in run_ids:
+                out[i].update(conv[i])
+        return out
 
-    def fit(self, data, silent=False):
-        """Fit ``sampling`` EM runs on a DataFrame with columns [users, items, ratings]."""
+    def fit(self, data, silent=False, tol=None, check_every=10):
+        """Fit ``sampling`` EM runs on a DataFrame with columns [users, items, ratings].
+
+        ``tol``: stop each run at convergence.  The observed-data log-likelihood (the quantity EM
+        increases) is evaluated at the start and every ``check_every`` steps (even, >= 2); a run stops
+        at the first check where it changed by at most ``tol`` times its magnitude since the previous
+        one, and ``self.iterations`` becomes the maximum.  Every ``results[s]`` then also holds
+        ``"iterations"`` (steps run), ``"converged"`` (False: stopped at the maximum) and ``"loglik"``
+        (the log-likelihood at each check up to the stop).  ``None`` (default): exactly
+        ``self.iterations`` steps, as before."""
+        self._check_convergence_args(tol, check_every)
         if not silent:
             self.logger.info(f"Running {self.sampling} runs of {self.iterations} iterations.")
         import time
@@ -268,7 +307,8 @@ class MMSBM:
         self._prepare_objects(train)
         self._tick("rows_h2d_index_build", t)
         mine = shard_runs(self.sampling, rank, world)
-        local = self._run_batch(self._engine, [self.child_states[i] for i in mine], mine) if mine else {}
+        local = self._run_batch(self._engine, [self.child_states[i] for i in mine], mine,
+                                tol=tol, check_every=check_every) if mine else {}
         self.results = gather_runs(local, self.sampling)
 
     def run_one_sampling(self, data, seed, i):
@@ -386,7 +426,7 @@ class MMSBM:
         return added
 
     # ------------------------------------------------------------------------ refit
-    def refit(self, data, iterations=None, seed=0):
+    def refit(self, data, iterations=None, seed=0, tol=None, check_every=10):
         """Fit on ``data`` again, starting from this model's parameters instead of random draws.
 
         ``data`` is the whole rating set the model should describe from now on -- normally the old
@@ -402,11 +442,15 @@ class MMSBM:
         a rating level without a row gets a zero pr slab, as in EM.  Calling ``fold_in(data)`` first
         gives the new ids a fold-in start instead of a random one.
 
+        ``tol`` / ``check_every``: stop each run at convergence, with ``iterations`` as the maximum
+        (see ``fit``).
+
         Afterwards ``results``, ``train`` and the degree factors describe ``data``, and
         ``likelihood`` / ``predict`` / ``score`` / ``save`` / ``refit`` work as after ``fit``.
         Returns {"users": [...], "items": [...]}: the labels added, in code order."""
         import time
         self._check_is_fitted()
+        self._check_convergence_args(tol, check_every)
         iterations = self.iterations if iterations is None else int(iterations)
         self.timings = {}
         t = time.perf_counter()
@@ -445,7 +489,7 @@ class MMSBM:
             self._tick("rows_h2d_index_build", t)
             mine = shard_runs(S, rank, world)
             local = self._run_batch(self._engine, None, mine, init=(theta0[mine], eta0[mine], pr0[mine]),
-                                    iterations=iterations) if mine else {}
+                                    iterations=iterations, tol=tol, check_every=check_every) if mine else {}
             # EM leaves a zero row where an id has no rating: put the old rows back, on the device too
             # when the engine still holds these runs for predict
             if self._resident is not None:
@@ -532,13 +576,15 @@ class MMSBM:
             alive[picked] = False
         return pairs
 
-    def cv_fit(self, data, folds=5):
+    def cv_fit(self, data, folds=5, tol=None, check_every=10):
         """k-fold cross-validation; returns the accuracy of every fold and keeps the objects of
         the most accurate one (src/mmsbm.py:371-472).  Under torch.distributed the folds x runs
-        jobs shard over the ranks (SURVEY.md section 8e.2); the result is the same."""
-        return self._cv_execute(self._make_folds(data, folds))
+        jobs shard over the ranks (SURVEY.md section 8e.2); the result is the same.  ``tol`` /
+        ``check_every``: every fit stops at convergence (see ``fit``)."""
+        self._check_convergence_args(tol, check_every)
+        return self._cv_execute(self._make_folds(data, folds), tol, check_every)
 
-    def _cv_execute(self, pairs):
+    def _cv_execute(self, pairs, tol=None, check_every=10):
         """Fit / predict / score every (train, test) pair and keep the best fold: the part of
         ``cv_fit`` after the fold construction (src/mmsbm.py:441-472)."""
         folds = len(pairs)
@@ -552,7 +598,8 @@ class MMSBM:
                 self.data_handler = DataHandler()
                 self._prepare_objects(self.data_handler.format_train_data(pairs[f][0]))
                 runs = [s for (ff, s) in mine if ff == f]
-                out = self._run_batch(self._engine, [self.child_states[s] for s in runs], runs)
+                out = self._run_batch(self._engine, [self.child_states[s] for s in runs], runs,
+                                      tol=tol, check_every=check_every)
                 local.update({(f, s): out[s] for s in runs})
             import torch.distributed as dist
             boxes = [None] * world
@@ -570,7 +617,7 @@ class MMSBM:
                 self._prepare_objects(self.data_handler.format_train_data(train), build_engine=False)
                 self.results = [done[(f, s)] for s in range(self.sampling)]
             else:
-                self.fit(train, silent=True)
+                self.fit(train, silent=True, tol=tol, check_every=check_every)
             self.prediction_matrix = self.predict(test)
             results = self.score(silent=True)
             all_results.append({
