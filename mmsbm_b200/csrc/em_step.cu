@@ -516,7 +516,7 @@ int sm_count() {
 // NCH 32-byte chunks per row are spread over G lanes x CH chunks per lane with G <= 8 (three
 // shuffle levels per rating at most); UN steps in flight; MINB CTAs per SM the kernel is
 // compiled for.  Defaults from the sweeps recorded in DESIGN.md section 5.
-static PassShape choose_shape(int NBp, double avg_degree) {
+static PassShape choose_shape(int NBp) {
   const int NCH = NBp / 4;
   int CH = 8;
   for (int c = 1; c <= 8; c *= 2) {
@@ -526,7 +526,6 @@ static PassShape choose_shape(int NBp, double avg_degree) {
   PassShape sh{G, CH, 1, 1};   // CH == 1 implies NBp == 4*G (the kernel relies on it)
   // three row loads in flight per warp, 3 CTAs/SM: best of the UN x MINB sweep on both passes
   // (four loads spill at 80 registers, 128 registers cost a third of the resident warps)
-  (void)avg_degree;
   if (CH == 1) { sh.UN = (G == 1) ? 1 : (G == 2) ? 2 : 3; sh.MINB = 3; }   // UN * (32 / G) <= 32
   else if (CH == 2) { sh.UN = 1; sh.MINB = 3; }
   return sh;
@@ -538,8 +537,6 @@ static PassShape choose_shape(int NBp, double avg_degree) {
 // warp to even out, long pieces want one per warp so that the last wave of CTAs is short -- and
 // at least ~6 CTAs per resident slot (148 SMs x 3) whatever the problem size.
 static int segs_per_cta_for(int64_t pmax, int64_t n_ratings, int grid_y) {
-  const int e = env_int("MMSBM_SPC", 0);
-  if (e > 0) return e;
   const double avg_piece = (double)(n_ratings > 0 ? n_ratings : 1) / (double)(pmax > 0 ? pmax : 1);
   int64_t spc = ((int64_t)(6144.0 / (avg_piece > 1.0 ? avg_piece : 1.0)) + kWarps / 2) / kWarps * kWarps;
   const int64_t fill = pmax * grid_y / (sm_count() * 3 * 6) / kWarps * kWarps;
@@ -552,7 +549,7 @@ static int segs_per_cta_for(int64_t pmax, int64_t n_ratings, int grid_y) {
 // pairs of runs per warp whenever there are at least two runs, a lane holds one chunk and the
 // w rows of a pair fit shared memory
 static bool pairs_enabled(int NBp, int R, int n_runs) {
-  return n_runs >= 2 && NBp <= 32 && seg_smem_bytes(R, NBp, 2) <= kMaxSmemBytes && env_int("MMSBM_PAIR", 1) != 0;
+  return n_runs >= 2 && NBp <= 32 && seg_smem_bytes(R, NBp, 2) <= kMaxSmemBytes;
 }
 
 // grid.x of a segment pass.  The piece count lives on the device, so the grid is sized for its upper
@@ -572,7 +569,7 @@ static unsigned grid_x_for(const SegArgs& a, int ctas_per_sm) {
 // six runs per warp: rows of exactly 20 doubles (5-lane groups, 30 of 32 lanes), at least six runs,
 // and the w rows of six runs fit shared memory (R <= 30)
 static bool hexa_enabled(int NBp, int R, int n_runs) {
-  return n_runs >= 6 && NBp == 20 && seg_smem_bytes(R, NBp, 6) <= kMaxSmemBytes && env_int("MMSBM_HEXA", 1) != 0;
+  return n_runs >= 6 && NBp == 20 && seg_smem_bytes(R, NBp, 6) <= kMaxSmemBytes;
 }
 
 RunPlan plan_runs(int NBp, int R, int n_runs, bool hexa_table) {
@@ -589,9 +586,7 @@ RunPlan plan_runs(int NBp, int R, int n_runs, bool hexa_table) {
 
 static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const double* nbr_hexa,
                                     int64_t n_ratings, int n_runs, cudaStream_t st) {
-  const double avg_degree = (double)n_ratings / (double)a.nseg;
-  PassShape sh = choose_shape(a.NBp, avg_degree);
-  const int un_e = env_int("MMSBM_UN", 0), occ_e = env_int("MMSBM_OCC", 0);
+  const PassShape sh = choose_shape(a.NBp);
   const RunPlan plan = plan_runs(a.NBp, a.R, n_runs, nbr_hexa != nullptr);
   const int single_from = plan.single_from;      // runs [single_from, n_runs) go one run per warp
   if (plan.hexas > 0) {
@@ -601,13 +596,10 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
     p.run_base = 0;
     p.grp_base = 0;
     p.segs_per_cta = segs_per_cta_for(a.pmax, n_ratings, hexas);
-    const unsigned gx = grid_x_for(p, occ_e > 0 ? occ_e : 3);
+    const unsigned gx = grid_x_for(p, 3);
     if (p.counters) a.counters += hexas;         // the next launch of this pass gets its own counters
     const size_t smem = seg_smem_bytes(a.R, a.NBp, 6);   // fits: plan_runs checked it
-    int rc = MMSBM_ERANGE;
-    if (un_e > 0 || occ_e > 0)
-      rc = launch_segment_pass_hexa(p, sh.G, un_e > 0 ? un_e : 3, occ_e > 0 ? occ_e : 3, dim3(gx, hexas), smem, st);
-    if (rc == MMSBM_ERANGE) rc = launch_segment_pass_hexa(p, sh.G, 3, 3, dim3(gx, hexas), smem, st);
+    const int rc = launch_segment_pass_hexa(p, sh.G, 3, 3, dim3(gx, hexas), smem, st);
     if (rc) {
       if (rc == MMSBM_ERANGE) set_error("no six-run segment-pass variant for G=%d", sh.G);
       return rc;
@@ -623,15 +615,11 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
     p.grp_base = plan.pair_group0;
     p.counters = a.counters;
     p.segs_per_cta = segs_per_cta_for(a.pmax, n_ratings, pairs);
-    const unsigned gx = grid_x_for(p, occ_e > 0 ? occ_e : 3);
+    const int UN = (sh.G == 1) ? 2 : 3, MINB = 3;               // UN * (32 / 2G) <= 32
+    const unsigned gx = grid_x_for(p, MINB);
     if (p.counters) a.counters += pairs;
     const size_t smem = seg_smem_bytes(a.R, a.NBp, 2);   // fits: plan_runs checked it
-    int UN = (sh.G == 1) ? 2 : 3, MINB = 3;                     // UN * (32 / 2G) <= 32
-    int rc = MMSBM_ERANGE;
-    if (un_e > 0 || occ_e > 0)
-      rc = launch_segment_pass_pair(p, sh.G, un_e > 0 ? un_e : UN, occ_e > 0 ? occ_e : MINB, dim3(gx, pairs), smem, st);
-    if (rc == MMSBM_ERANGE) rc = launch_segment_pass_pair(p, sh.G, UN, MINB, dim3(gx, pairs), smem, st);
-    if (rc == MMSBM_ERANGE && sh.G == 1) rc = launch_segment_pass_pair(p, sh.G, 2, 3, dim3(gx, pairs), smem, st);
+    const int rc = launch_segment_pass_pair(p, sh.G, UN, MINB, dim3(gx, pairs), smem, st);
     if (rc) {
       if (rc == MMSBM_ERANGE) set_error("no paired segment-pass variant for G=%d", sh.G);
       return rc;
@@ -640,28 +628,18 @@ static int launch_segment_pass_impl(SegArgs a, const double* nbr_pairs, const do
   if (single_from == n_runs) return 0;
   a.run_base = single_from;
   a.segs_per_cta = segs_per_cta_for(a.pmax, n_ratings, n_runs - single_from);
-  const unsigned gx = grid_x_for(a, occ_e > 0 ? occ_e : sh.MINB);
+  const unsigned gx = grid_x_for(a, sh.MINB);
   const dim3 grid(gx, n_runs - single_from);
   const size_t smem = seg_smem_bytes(a.R, a.NBp, 1);
   MMSBM_REQUIRE(smem <= kMaxSmemBytes, MMSBM_ERANGE,
                 "segment pass needs %zu bytes of shared memory (R=%d, row stride %d)", smem, a.R, a.NBp);
-  auto go = [&](const PassShape& p) {
-    switch (p.CH) {
-      case 1: return launch_segment_pass_ch1(a, p.G, p.UN, p.MINB, grid, smem, st);
-      case 2: return launch_segment_pass_ch2(a, p.G, p.UN, p.MINB, grid, smem, st);
-      case 4: return launch_segment_pass_ch4(a, p.G, p.UN, p.MINB, grid, smem, st);
-      default: return launch_segment_pass_ch8(a, p.G, p.UN, p.MINB, grid, smem, st);
-    }
-  };
-  // tuning overrides (only combinations that were instantiated take effect)
-  if (un_e > 0 || occ_e > 0) {
-    PassShape alt = sh;
-    if (un_e > 0) alt.UN = un_e;
-    if (occ_e > 0) alt.MINB = occ_e;
-    const int rc = go(alt);
-    if (rc != MMSBM_ERANGE) return rc;
+  int rc;
+  switch (sh.CH) {
+    case 1: rc = launch_segment_pass_ch1(a, sh.G, sh.UN, sh.MINB, grid, smem, st); break;
+    case 2: rc = launch_segment_pass_ch2(a, sh.G, sh.UN, sh.MINB, grid, smem, st); break;
+    case 4: rc = launch_segment_pass_ch4(a, sh.G, sh.UN, sh.MINB, grid, smem, st); break;
+    default: rc = launch_segment_pass_ch8(a, sh.G, sh.UN, sh.MINB, grid, smem, st); break;
   }
-  const int rc = go(sh);
   if (rc == MMSBM_ERANGE) set_error("no segment-pass variant for G=%d CH=%d UN=%d", sh.G, sh.CH, sh.UN);
   return rc;
 }
@@ -713,14 +691,12 @@ static int launch_gemm(GemmArgs g, int n_runs, cudaStream_t st) {
 int launch_w(const double* own, const double* pw, double* W, int M, int LD, int RNB, int n_runs,
              cudaStream_t st) {
   const size_t smem = (size_t)LD * RNB * 8;
-  const int rows_env = env_int("MMSBM_ROWS", 2);
 #define MMSBM_ROW_W(LDv)                                                                        \
   if (LD == LDv && smem <= 200 * 1024) {                                                        \
     constexpr int kRows = (LDv <= 24) ? 2 : 1;   /* 2 x LD operand registers per lane */          \
-    const bool two = kRows == 2 && rows_env == 2;                                               \
-    auto kern = two ? row_w_kernel<LDv, kRows> : row_w_kernel<LDv, 1>;                          \
-    const int per = kRowThreads * (two ? 2 : 1);                                                \
-    const int gx = min((M + per - 1) / per, sm_count() * 2);                                           \
+    auto kern = row_w_kernel<LDv, kRows>;                                                       \
+    const int per = kRowThreads * kRows;                                                        \
+    const int gx = min((M + per - 1) / per, sm_count() * 2);                                    \
     MMSBM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     kern<<<dim3(gx, n_runs), kRowThreads, smem, st>>>(own, pw, W, M, RNB);                      \
     MMSBM_LAUNCH_CHECK("row_w_kernel");                                                         \
@@ -738,16 +714,12 @@ int launch_n(const double* G, const double* pn, const double* own, const int32_t
   const size_t smem = (size_t)LD * RNB * 8;
   RowPublish pub{};
   if (publish) pub = *publish;
-  // one row per lane here: two rows cost occupancy (142 registers) and measured slower
-  const int rows_env = env_int("MMSBM_ROWS_N", 1);
-  // chunks in flight per lane: MMSBM_ROWN_PF (1 = round-1 behaviour); needs (RNB / 4) % PF == 0
-  int pf = env_int("MMSBM_ROWN_PF", 5);
-  if (pf != 1 && pf != 2 && pf != 5) pf = 1;
-  if ((RNB / 4) % pf != 0) pf = ((RNB / 4) % 2 == 0 && pf != 1) ? 2 : 1;
-#define MMSBM_ROW_N_GO(kern, two)                                                               \
+  // one row per lane here: two rows cost occupancy (142 registers) and measured slower.  PF chunks
+  // of the G row in flight per lane; PF must divide RNB / 4
+  const int pf = (RNB / 4) % 5 == 0 ? 5 : (RNB / 4) % 2 == 0 ? 2 : 1;
+#define MMSBM_ROW_N_GO(kern)                                                                    \
   {                                                                                             \
-    const int per = kRowThreads * ((two) ? 2 : 1);                                              \
-    const int gx = min((M + per - 1) / per, sm_count() * 2);                                    \
+    const int gx = min((M + kRowThreads - 1) / kRowThreads, sm_count() * 2);                    \
     MMSBM_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)); \
     kern<<<dim3(gx, n_runs), kRowThreads, smem, st>>>(G, pn, own, deg, out, M, RNB, normalize, pub); \
     MMSBM_LAUNCH_CHECK("row_n_kernel");                                                         \
@@ -755,12 +727,9 @@ int launch_n(const double* G, const double* pn, const double* own, const int32_t
   }
 #define MMSBM_ROW_N(LDv)                                                                        \
   if (LD == LDv && smem <= 200 * 1024) {                                                        \
-    constexpr int kRows = (LDv <= 24) ? 2 : 1;   /* 2 x LD accumulator registers per lane */      \
-    const bool two = kRows == 2 && rows_env == 2;                                               \
-    if (two) MMSBM_ROW_N_GO((row_n_kernel<LDv, kRows, 1>), true)                                \
-    if (pf == 5) MMSBM_ROW_N_GO((row_n_kernel<LDv, 1, 5>), false)                               \
-    if (pf == 2) MMSBM_ROW_N_GO((row_n_kernel<LDv, 1, 2>), false)                               \
-    MMSBM_ROW_N_GO((row_n_kernel<LDv, 1, 1>), false)                                            \
+    if (pf == 5) MMSBM_ROW_N_GO((row_n_kernel<LDv, 1, 5>))                                      \
+    if (pf == 2) MMSBM_ROW_N_GO((row_n_kernel<LDv, 1, 2>))                                      \
+    MMSBM_ROW_N_GO((row_n_kernel<LDv, 1, 1>))                                                   \
   }
   MMSBM_ROW_N(4) MMSBM_ROW_N(8) MMSBM_ROW_N(12) MMSBM_ROW_N(16) MMSBM_ROW_N(20) MMSBM_ROW_N(24)
   MMSBM_ROW_N(28) MMSBM_ROW_N(32)

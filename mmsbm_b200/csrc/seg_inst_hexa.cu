@@ -2,8 +2,7 @@
 #include "segment_pass.cuh"
 namespace mmsbm {
 int launch_segment_pass_hexa(const SegArgs& a, int G, int UN, int MINB, dim3 grid, size_t smem, cudaStream_t st) {
-  MMSBM_SEG_LAUNCH_R(5, 1, 3, 3, 6) MMSBM_SEG_LAUNCH_R(5, 1, 4, 3, 6) MMSBM_SEG_LAUNCH_R(5, 1, 2, 4, 6)
-  MMSBM_SEG_LAUNCH_R(5, 1, 4, 2, 6) MMSBM_SEG_LAUNCH_R(5, 1, 6, 2, 6)
+  MMSBM_SEG_LAUNCH_R(5, 1, 3, 3, 6)
   return MMSBM_ERANGE;
 }
 }  // namespace mmsbm

@@ -462,12 +462,11 @@ extern "C" int mmsbm_em_run_sharded(const mmsbm_shard_t* shp, int32_t iterations
   // pieces a warp gets only a few, and claiming them dynamically evens the tails out (measured on one
   // rank's share of ML-20M / 8: 0.907 -> 0.897 ms per iteration)
   const bool dyn = env_int("MMSBM_DYN", n_big >= ((int64_t)1 << 20) ? 1 : 0) != 0;
-  const bool alternate = peers && env_int("MMSBM_SHARD_ALTERNATE", 1) != 0;
-  const bool overlap = peers && env_int("MMSBM_SHARD_OVERLAP", 1) != 0;   // aux stream beside the main one
-  const bool fuse = env_int("MMSBM_SHARD_FUSE", 1) != 0;   // row_n_kernel writes the table slice itself
+  const bool alternate = peers;
+  const bool overlap = peers;                   // aux stream beside the main one
   // persistent CTAs of the passes leave a few slots free so that the NCCL kernels of the side stream
   // can start while a pass runs
-  if (peers) set_reserved_ctas(env_int("MMSBM_SHARD_RESERVE", 4));
+  if (peers) set_reserved_ctas(4);
   const void* mine = sh.exchange_dev[sh.rank];
   if (peers) {                                  // the side stream starts behind everything queued on `st`
     MMSBM_CUDA(cudaEventRecord(ex.partial, st));
@@ -501,9 +500,9 @@ extern "C" int mmsbm_em_run_sharded(const mmsbm_shard_t* shp, int32_t iterations
     //  slice of the next gather tables -- no separate interleave pass)
     auto finish_users = [&](cudaStream_t fs) -> int {
       const RowPublish pub = row_publish(mine, g, g.theta, 2, nxt, sh.n_users, sh.user_lo);
-      int r = launch_n(wg_u, pn_u, th, sh.udeg_dev, th_n, Uo, d.ldk, d.rnb_u, 1, S, fs, fuse ? &pub : nullptr);
+      int r = launch_n(wg_u, pn_u, th, sh.udeg_dev, th_n, Uo, d.ldk, d.rnb_u, 1, S, fs, &pub);
       if (r) return r;
-      return publish_side(sh, g, g.theta, 2, fuse ? nullptr : th_n, Uo, sh.user_lo, nxt, fs, ex);
+      return publish_side(sh, g, g.theta, 2, nullptr, Uo, sh.user_lo, nxt, fs, ex);
     };
     auto pass_items = [&]() -> int {            // gathers theta rows of ALL users, new eta rows of the own items
       if (have_arrival[0]) MMSBM_CUDA(cudaStreamWaitEvent(st, ex.arrived[0][(it + 1) & 1], 0));
@@ -513,9 +512,9 @@ extern "C" int mmsbm_em_run_sharded(const mmsbm_shard_t* shp, int32_t iterations
     };
     auto finish_items = [&](cudaStream_t fs) -> int {
       const RowPublish pub = row_publish(mine, g, g.eta, 3, nxt, sh.n_items, sh.item_lo);
-      int r = launch_n(wg_i, pn_i, et, sh.ideg_dev, et_n, Io, d.ldl, d.rnb_i, 1, S, fs, fuse ? &pub : nullptr);
+      int r = launch_n(wg_i, pn_i, et, sh.ideg_dev, et_n, Io, d.ldl, d.rnb_i, 1, S, fs, &pub);
       if (r) return r;
-      return publish_side(sh, g, g.eta, 3, fuse ? nullptr : et_n, Io, sh.item_lo, nxt, fs, ex);
+      return publish_side(sh, g, g.eta, 3, nullptr, Io, sh.item_lo, nxt, fs, ex);
     };
     auto reduce_pr = [&](cudaStream_t fs) -> int {   // partial n_pr on fs, its sum over the ranks on the side stream
       int r = launch_pr(emit_items ? et : th, emit_items ? wg_i : wg_u, partial, pr, pr_n, emit_items ? Io : Uo,

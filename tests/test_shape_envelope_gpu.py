@@ -9,10 +9,13 @@ file runs the edges of that envelope through each of them:
   largest admitted R and at R = 5, with run counts that reach the pair and six-run groupings),
   comparing one EM step, the likelihood, the rating distributions and fold-in with the oracle;
 * end-to-end fits at shapes whose sizes sit at the shared-memory limits;
-* a coverage check: every kernel variant the default dispatch can pick is launched by the sweep.
+* a coverage check: every kernel variant the default dispatch can pick is launched by the sweep, and
+  the library holds no segment-pass instance the dispatch cannot pick.
 
 The shapes come from ``_check_shape`` itself, so the sweep follows the rule if it ever changes."""
+import os
 import re
+import subprocess
 
 import numpy as np
 import pandas as pd
@@ -230,7 +233,8 @@ def test_sharded_engine_one_rank_at_the_pair_limit():
 
 # ---------------------------------------------------------------------------------- coverage
 # Every variant the default dispatch can pick.  A kernel or an instance added to the library
-# belongs in this list, and the sweep must reach it.
+# belongs in this list, and the sweep must reach it; the segment-pass instances in the library are
+# exactly SEGMENT_PASS.
 SEGMENT_PASS = (
     # one run per warp: ld 4, 8, 12..32 (one chunk per lane), then 2 / 4 / 8 chunks per lane
     ["segment_pass_kernel<1,1,1,3,1>", "segment_pass_kernel<2,1,2,3,1>"]
@@ -251,6 +255,18 @@ EXPECTED = (SEGMENT_PASS
                "prod_dist_kernel<0>", "prod_dist_kernel<1>"])
 
 
+def library_segment_pass_instances():
+    """'segment_pass_kernel<G,CH,UN,MINB,RUNS>' of every instance in the library _lib loads, read from
+    the mangled names that `cuobjdump -symbols` lists."""
+    from mmsbm_b200 import _lib
+    from mmsbm_b200.build import _nvcc
+    nvcc = _nvcc()
+    tool = os.path.join(os.path.dirname(nvcc), "cuobjdump") if os.path.isabs(nvcc) else "cuobjdump"
+    out = subprocess.run([tool, "-symbols", _lib.LIB_PATH], capture_output=True, text=True, check=True).stdout
+    return {"segment_pass_kernel<%s>" % ",".join(re.findall(r"Li(\d+)E", args))
+            for args in re.findall(r"segment_pass_kernelI((?:Li\d+E)+)E", out)}
+
+
 def normalise(name):
     """'void mmsbm::segment_pass_kernel<(int)5, (int)1, ...>(mmsbm::SegArgs)' -> 'segment_pass_kernel<5,1,...>'"""
     name = re.sub(r"\((?:int|bool)\)|\s", "", name).replace("true", "1").replace("false", "0")
@@ -268,3 +284,8 @@ def test_sweep_launches_every_kernel_variant():
     launched = {normalise(ev.key) for ev in prof.key_averages()}
     missing = [k for k in EXPECTED if not any(n.startswith(k) for n in launched)]
     assert not missing, missing
+    # the reverse: an instance the dispatch cannot pick is code no test runs
+    built = library_segment_pass_instances()
+    assert built, "no segment_pass_kernel symbol found"
+    extra = sorted(built - set(SEGMENT_PASS))
+    assert not extra, extra
