@@ -252,7 +252,9 @@ int mmsbm_em_run_sharded(const mmsbm_shard_t* shard, int32_t iterations,
  *      (src/expectation_maximization.py:157-167); out_dev[S] ------------------------------ */
 /* usched_dev: the by-user work schedule of mmsbm_graph_build.  With it (and rows of at most 32
  * doubles) the sum is evaluated in its factorised form, O(K+L) per rating; NULL selects the
- * element-wise form, K*L visits per rating.  The runs are processed in batches that fit the
+ * element-wise form, K*L visits per rating.  A run where the factorised form's bound on the
+ * reference's eps clamps exceeds 1e-9 of its total (one-hot memberships of a converged fit) is
+ * evaluated again element-wise, decided on the device.  The runs are processed in batches that fit the
  * workspace: _workspace_bytes = all runs at once, _min_workspace_bytes = one run at a time. */
 int mmsbm_likelihood_workspace_bytes(int64_t n_ratings, int32_t n_users, int32_t n_items, int32_t n_levels,
                                      int32_t K, int32_t L, int32_t n_runs, size_t* bytes);

@@ -29,13 +29,14 @@ struct LikArgs {
   double* partial;      // [S][kLikCtas*kLikWarps]
   double* tables;       // [S][2][R][K][L] in global memory when they do not fit shared memory
   int U, I, R, K, L, ldk, ldl;
+  const int* redo;      // [S] or null: only the runs with redo[run] != 0 are evaluated
 };
 
 // pr and log pr in [R][K][L] order (global-memory variant of the tables)
-__global__ void lik_tables_kernel(const double* pr, int K, int L, int R, double* tables) {
+__global__ void lik_tables_kernel(const double* pr, int K, int L, int R, double* tables, const int* redo) {
   const int run = blockIdx.y, n = K * L * R;
   const int t = blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n) return;
+  if (t >= n || (redo && !redo[run])) return;
   const int kl = t / R, r = t - kl * R;
   const double v = __ldg(pr + (size_t)run * n + t);
   double* base = tables + (size_t)run * 2 * n;
@@ -49,6 +50,7 @@ __global__ void __launch_bounds__(kLikWarps * 32) likelihood_kernel(const LikArg
   const double kLogEps = log(kEps);
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int run = blockIdx.y;
+  if (A.redo && !A.redo[run]) return;                        // the factorised total of this run stands
   const double* Pq;                                          // [R][K][L]
   const double* Lq;                                          // [R][K][L]  log pr
   double* th_s;                                              // [warps][2][K]  theta, log theta
@@ -128,11 +130,15 @@ __global__ void __launch_bounds__(kLikWarps * 32) likelihood_kernel(const LikArg
 //     likelihood = sum_n T_n - S_n log max(S_n, eps)
 // i.e. O(K+L) per rating after two per-(user, level) tables, instead of K*L element visits and
 // L logarithms.  x log x := 0 at x = 0.  The reference clamps every w below eps up to eps
-// (src/expectation_maximization.py:162-166); here such an element contributes w log w instead of
-// eps log eps: at most 8e-15 per element, i.e. <= 1e-11 relative on the totals of interest,
-// inside the 1e-8 the likelihood is specified to (north_star).  Walks the (user, level)-grouped
-// index with the piece schedule of the EM step, so a heavy user costs no more than 2048 ratings
-// per warp; one partial per piece, summed in piece order.
+// (src/expectation_maximization.py:162-166); here such an element contributes w (log w - log S~)
+// instead of eps (log eps - log S~), a difference of at most eps (2 |log eps| + |log S~_n|).  Over
+// a run that is at most K L eps (2 N |log eps| + sum_n |log S~_n|), which the pass bounds by also
+// summing |log S~_n|.  On dense parameters the bound is ~1e-12 relative to the total; on a
+// converged fit with one-hot memberships the total itself shrinks toward 0 and is made of clamp
+// terms, and the factorised form can be off by 100 %.  So a run whose bound exceeds 1e-9 of its
+// factorised total is evaluated again by likelihood_kernel (decided on the device, lik_check_kernel).
+// Walks the (user, level)-grouped index with the piece schedule of the EM step, so a heavy user
+// costs no more than 2048 ratings per warp; one partial per piece, summed in piece order.
 __device__ __forceinline__ double xlogx(double x) { return x > 0.0 ? x * log(x) : 0.0; }
 
 // E2[run][item][0][:] = eta, [1][:] = eta log eta  (one contiguous 2*8*ldl-byte gather per rating)
@@ -203,6 +209,7 @@ struct LikPassArgs {
   int64_t pmax;
   int U, I, R;
   int ld;                 // OBS: row stride of eta (NBp when G < 8, any multiple of 4 >= 32 when G == 8)
+  double* lpartial;       // [runs][pmax] sum_n |log S~_n| of the piece (not written by OBS)
 };
 
 // One warp per piece; groups of G lanes own a rating (lane q holds doubles 4q..4q+3 of both rows).
@@ -234,7 +241,7 @@ __device__ __forceinline__ void lik_pass_body(const LikPassArgs& P) {
     const int end = min(beg + MMSBM_PIECE_LEN, __shfl_sync(kFull, bend, R));
     const double* wrow = P.W + ((size_t)run * P.U + sg) * RNB;
     const double* arow = P.A + ((size_t)run * P.U + sg) * RNB;
-    double acc = 0.0;
+    double acc = 0.0, lacc = 0.0;
     int lo = beg;
     for (int r = 0; r < R; ++r) {
       const int le = min(end, __shfl_sync(kFull, bend, r + 1));
@@ -296,13 +303,21 @@ __device__ __forceinline__ void lik_pass_body(const LikPassArgs& P) {
           t = fma(el[un].x, wr.x, fma(el[un].y, wr.y, fma(el[un].z, wr.z, fma(el[un].w, wr.w, t))));
           s = group_sum(s);
           t = group_sum(t);
-          if (lane_on && q == 0 && un * RPS + grp < cnt) acc += t - s * log(fmax(s, kEps));
+          if (lane_on && q == 0 && un * RPS + grp < cnt) {
+            const double ls = log(fmax(s, kEps));
+            acc += t - s * ls;
+            lacc += fabs(ls);
+          }
         }
       }
       lo = le;
     }
     acc = warp_sum(acc);
     if (lane == 0) P.partial[(size_t)run * P.pmax + p] = acc;
+    if constexpr (!OBS) {
+      lacc = warp_sum(lacc);
+      if (lane == 0) P.lpartial[(size_t)run * P.pmax + p] = lacc;
+    }
   }
 }
 
@@ -312,7 +327,11 @@ __global__ void __launch_bounds__(256) lik_pass_kernel(const LikPassArgs P) { li
 template <int G>
 __global__ void __launch_bounds__(256) loglik_pass_kernel(const LikPassArgs P) { lik_pass_body<G, true>(P); }
 
-__global__ void __launch_bounds__(256) sum_partials_kernel(const double* partial, int n, double* out) {
+// out[run] = the fixed-order sum of the run's n partials (only the runs with only[run] != 0 when
+// only is given)
+__global__ void __launch_bounds__(256) sum_partials_kernel(const double* partial, int n, double* out,
+                                                           const int* only = nullptr) {
+  if (only && !only[blockIdx.x]) return;
   __shared__ double sm[256];
   const double* p = partial + (size_t)blockIdx.x * n;
   double acc = 0.0;
@@ -324,6 +343,16 @@ __global__ void __launch_bounds__(256) sum_partials_kernel(const double* partial
     __syncthreads();
   }
   if (threadIdx.x == 0) out[blockIdx.x] = sm[0];
+}
+
+// redo[run] = 1 when what the clamps the factorised form drops could move the run's total by more
+// than 1e-9 of it: K L eps (2 N |log eps| + sum_n |log S~_n|) > 1e-9 |total| (NaN totals included)
+__global__ void lik_check_kernel(const double* total, const double* labs, int S, double kl_eps,
+                                 double two_n_logeps, int* redo) {
+  const int run = blockIdx.x * blockDim.x + threadIdx.x;
+  if (run >= S) return;
+  const double bound = kl_eps * (two_n_logeps + labs[run]);
+  redo[run] = !(bound <= 1e-9 * fabs(total[run]));
 }
 
 // ---- prod_dist -----------------------------------------------------------------------------
@@ -481,6 +510,15 @@ using namespace mmsbm;
 // [2][R][K][L] tables of one run of the element-wise likelihood (global memory when they do not fit
 // shared memory)
 static size_t lik_table_bytes(int R, int K, int L) { return 2 * (size_t)R * K * L * 8; }
+// the element-wise kernel keeps its two tables in global memory when they and the theta rows of its
+// warps do not fit 200 KB of shared memory
+static size_t lik_elementwise_smem(int R, int K, int L) { return (2 * (size_t)R * K * L + 2 * (size_t)kLikWarps * K) * 8; }
+static bool lik_elementwise_tables(int R, int K, int L) { return lik_elementwise_smem(R, K, L) > 200 * 1024; }
+// what the element-wise evaluation takes from the workspace (partials, and tables when it needs them)
+static size_t lik_elementwise_bytes(int R, int K, int L, int S) {
+  return align_up((size_t)S * kLikCtas * kLikWarps * 8) +
+         (lik_elementwise_tables(R, K, L) ? align_up((size_t)S * lik_table_bytes(R, K, L)) : 0);
+}
 
 static int lik_env_int(const char* name, int dflt) {
   const char* v = getenv(name);
@@ -499,15 +537,23 @@ static size_t lik_run_bytes(int U, int I, int R, int L) {      // tables of one 
   return 2 * align_up((size_t)U * rnb * 8) + align_up((size_t)I * 2 * ldl * 8);
 }
 static int64_t lik_pmax(int64_t N, int U) { return (int64_t)U + N / MMSBM_PIECE_LEN + 1; }   // = graph_build.cu
+// the factorised path's fixed part: two partials per piece, the per-run |log S~| sum and redo flag,
+// and room for the element-wise evaluation of the runs it hands over.  Its tables are usually in
+// shared memory, but not always: K = 16, L = 32, R = 25 passes lik_factorised_ok (16 R ldk ldl =
+// 200 KB) while the element-wise kernel also needs 2 K doubles per warp.
+static size_t lik_fact_fixed_bytes(int64_t N, int U, int R, int K, int L, int S) {
+  return 2 * align_up((size_t)S * lik_pmax(N, U) * 8) + align_up((size_t)S * 8) + align_up((size_t)S * 4) +
+         lik_elementwise_bytes(R, K, L, S);
+}
 
 extern "C" int mmsbm_likelihood_workspace_bytes(int64_t N, int32_t U, int32_t I, int32_t R, int32_t K,
                                                 int32_t L, int32_t S, size_t* bytes) {
   MMSBM_REQUIRE(bytes && N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
                 "mmsbm_likelihood_workspace_bytes: bad argument");
-  const size_t elementwise = align_up((size_t)S * kLikCtas * kLikWarps * 8) + align_up((size_t)S * lik_table_bytes(R, K, L)) + 256;
+  const size_t elementwise = lik_elementwise_bytes(R, K, L, S) + 256;
   size_t fact = 0;
   if (lik_factorised_ok(R, K, L))
-    fact = align_up((size_t)S * lik_pmax(N, U) * 8) + (size_t)S * lik_run_bytes(U, I, R, L) + 256;
+    fact = lik_fact_fixed_bytes(N, U, R, K, L, S) + (size_t)S * lik_run_bytes(U, I, R, L) + 256;
   *bytes = fact > elementwise ? fact : elementwise;
   return 0;
 }
@@ -517,11 +563,37 @@ extern "C" int mmsbm_likelihood_min_workspace_bytes(int64_t N, int32_t U, int32_
                                                     int32_t L, int32_t S, size_t* bytes) {
   MMSBM_REQUIRE(bytes && N >= 0 && U > 0 && I > 0 && R > 0 && K > 0 && L > 0 && S > 0, MMSBM_EINVAL,
                 "mmsbm_likelihood_min_workspace_bytes: bad argument");
-  const size_t elementwise = align_up((size_t)S * kLikCtas * kLikWarps * 8) + align_up((size_t)S * lik_table_bytes(R, K, L)) + 256;
+  const size_t elementwise = lik_elementwise_bytes(R, K, L, S) + 256;
   size_t fact = 0;
   if (lik_factorised_ok(R, K, L))
-    fact = align_up((size_t)S * lik_pmax(N, U) * 8) + lik_run_bytes(U, I, R, L) + 256;
+    fact = lik_fact_fixed_bytes(N, U, R, K, L, S) + lik_run_bytes(U, I, R, L) + 256;
   *bytes = fact > elementwise ? fact : elementwise;
+  return 0;
+}
+
+// Element-wise form: K*L visits per rating, partials and (when they do not fit shared memory)
+// tables taken from the arena.  With redo, only the runs flagged there are evaluated and written.
+static int likelihood_elementwise(Arena& arena, const int32_t* useg, const int32_t* uadj, int U, int I, int R,
+                                  int K, int L, int S, const double* theta, const double* eta, const double* pr,
+                                  double* out, const int* redo, cudaStream_t st) {
+  const int nw = kLikCtas * kLikWarps;
+  double* partial = arena.take<double>((size_t)S * nw);
+  MMSBM_REQUIRE(partial, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
+  LikArgs a{useg, uadj, theta, eta, pr, partial, nullptr, U, I, R, K, L, row_stride(K), row_stride(L), redo};
+  size_t smem = lik_elementwise_smem(R, K, L);
+  if (lik_elementwise_tables(R, K, L)) {         // keep the two tables in global memory (L2 resident)
+    a.tables = arena.take<double>((size_t)S * lik_table_bytes(R, K, L) / 8);
+    MMSBM_REQUIRE(a.tables, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
+    const int n = K * L * R;
+    lik_tables_kernel<<<dim3((n + 255) / 256, S), 256, 0, st>>>(pr, K, L, R, a.tables, redo);
+    MMSBM_LAUNCH_CHECK("lik_tables_kernel");
+    smem = 2 * (size_t)kLikWarps * K * 8;
+  }
+  MMSBM_CUDA(cudaFuncSetAttribute(likelihood_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  likelihood_kernel<<<dim3(kLikCtas, S), kLikWarps * 32, smem, st>>>(a);
+  MMSBM_LAUNCH_CHECK("likelihood_kernel");
+  sum_partials_kernel<<<S, 256, 0, st>>>(partial, nw, out, redo);
+  MMSBM_LAUNCH_CHECK("sum_partials_kernel");
   return 0;
 }
 
@@ -544,11 +616,16 @@ static int likelihood_factorised(const int32_t* useg, const int32_t* uadj, const
   const int ldk = row_stride(K), ldl = row_stride(L);
   const size_t rnb = (size_t)R * ldl;
   const int64_t pmax = lik_pmax(N, U);
+  MMSBM_REQUIRE(pmax <= 0x7fffffff, MMSBM_ERANGE, "mmsbm_likelihood: too many pieces");
   Arena arena(ws, ws_bytes);
   double* partial = arena.take<double>((size_t)S * pmax);
-  MMSBM_REQUIRE(partial, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
-  const size_t per_run = lik_run_bytes(U, I, R, L);
-  int nb = (int)((ws_bytes - arena.off) / per_run);          // runs per batch that fit the workspace
+  double* lpartial = arena.take<double>((size_t)S * pmax);
+  double* labs = arena.take<double>(S);
+  int* redo = arena.take<int>(S);
+  MMSBM_REQUIRE(partial && lpartial && labs && redo, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
+  const size_t per_run = lik_run_bytes(U, I, R, L), reserved = lik_elementwise_bytes(R, K, L, S);
+  // runs per batch that fit the workspace next to what the element-wise evaluation takes
+  int nb = ws_bytes - arena.off >= reserved ? (int)((ws_bytes - arena.off - reserved) / per_run) : 0;
   if (nb > S) nb = S;
   MMSBM_REQUIRE(nb >= 1, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small for one run (%zu bytes)", ws_bytes);
   double* W = arena.take<double>((size_t)nb * U * rnb);
@@ -556,6 +633,7 @@ static int likelihood_factorised(const int32_t* useg, const int32_t* uadj, const
   double* e2 = arena.take<double>((size_t)nb * I * 2 * ldl);
   MMSBM_REQUIRE(W && A && e2, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
   MMSBM_CUDA(cudaMemsetAsync(partial, 0, (size_t)S * pmax * 8, st));
+  MMSBM_CUDA(cudaMemsetAsync(lpartial, 0, (size_t)S * pmax * 8, st));
   for (int run0 = 0; run0 < S; run0 += nb) {
     const int n = S - run0 < nb ? S - run0 : nb;
     {
@@ -575,7 +653,8 @@ static int likelihood_factorised(const int32_t* useg, const int32_t* uadj, const
       case 32: rc = launch_lik_tables<32>(theta, pr, W, A, U, K, L, R, run0, n, st); break;
     }
     if (rc) return rc;
-    LikPassArgs a{useg, uadj, usched, e2, W, A, partial + (size_t)run0 * pmax, pmax, U, I, R, ldl};
+    LikPassArgs a{useg, uadj, usched, e2, W, A, partial + (size_t)run0 * pmax, pmax, U, I, R, ldl,
+                  lpartial + (size_t)run0 * pmax};
     const int64_t want = (pmax + 7) / 8;
     const int64_t cap = (int64_t)sm_count() * 16;
     const dim3 grid((unsigned)(want < cap ? want : cap), n);
@@ -591,10 +670,15 @@ static int likelihood_factorised(const int32_t* useg, const int32_t* uadj, const
     }
     MMSBM_LAUNCH_CHECK("lik_pass_kernel");
   }
-  MMSBM_REQUIRE(pmax <= 0x7fffffff, MMSBM_ERANGE, "mmsbm_likelihood: too many pieces");
   sum_partials_kernel<<<S, 256, 0, st>>>(partial, (int)pmax, out);
   MMSBM_LAUNCH_CHECK("sum_partials_kernel");
-  return 0;
+  sum_partials_kernel<<<S, 256, 0, st>>>(lpartial, (int)pmax, labs);
+  MMSBM_LAUNCH_CHECK("sum_partials_kernel");
+  lik_check_kernel<<<(S + 127) / 128, 128, 0, st>>>(out, labs, S, (double)K * L * kEps, -2.0 * (double)N * log(kEps),
+                                                     redo);
+  MMSBM_LAUNCH_CHECK("lik_check_kernel");
+  // the runs the bound does not clear: the element-wise form, whose bits replace the factorised total
+  return likelihood_elementwise(arena, useg, uadj, U, I, R, K, L, S, theta, eta, pr, out, redo, st);
 }
 
 extern "C" int mmsbm_likelihood(const int32_t* useg, const int32_t* uadj, const int32_t* usched, int64_t N,
@@ -608,27 +692,9 @@ extern "C" int mmsbm_likelihood(const int32_t* useg, const int32_t* uadj, const 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (usched && lik_factorised_ok(R, K, L))
     return likelihood_factorised(useg, uadj, usched, N, U, I, R, K, L, S, theta, eta, pr, out, ws, ws_bytes, st);
-  // element-wise path (rows wider than 32 doubles, or no schedule given): K*L visits per rating
+  // element-wise path (rows wider than 32 doubles, or no schedule given)
   Arena arena(ws, ws_bytes);
-  const int nw = kLikCtas * kLikWarps;
-  double* partial = arena.take<double>((size_t)S * nw);
-  MMSBM_REQUIRE(partial, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
-  LikArgs a{useg, uadj, theta, eta, pr, partial, nullptr, U, I, R, K, L, row_stride(K), row_stride(L)};
-  size_t smem = (2 * (size_t)R * K * L + 2 * (size_t)kLikWarps * K) * 8;
-  if (smem > 200 * 1024) {                       // keep the two tables in global memory (L2 resident)
-    a.tables = arena.take<double>((size_t)S * lik_table_bytes(R, K, L) / 8);
-    MMSBM_REQUIRE(a.tables, MMSBM_ENOMEM, "mmsbm_likelihood: workspace too small");
-    const int n = K * L * R;
-    lik_tables_kernel<<<dim3((n + 255) / 256, S), 256, 0, st>>>(pr, K, L, R, a.tables);
-    MMSBM_LAUNCH_CHECK("lik_tables_kernel");
-    smem = 2 * (size_t)kLikWarps * K * 8;
-  }
-  MMSBM_CUDA(cudaFuncSetAttribute(likelihood_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  likelihood_kernel<<<dim3(kLikCtas, S), kLikWarps * 32, smem, st>>>(a);
-  MMSBM_LAUNCH_CHECK("likelihood_kernel");
-  sum_partials_kernel<<<S, 256, 0, st>>>(partial, nw, out);
-  MMSBM_LAUNCH_CHECK("sum_partials_kernel");
-  return 0;
+  return likelihood_elementwise(arena, useg, uadj, U, I, R, K, L, S, theta, eta, pr, out, nullptr, st);
 }
 
 // ---- observed-data log-likelihood ----------------------------------------------------------
